@@ -9,6 +9,7 @@ Matern-5/2 ARD, 1024 MC samples, sum-of-squares composite), 1M candidates per GP
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          our CUDA path (one JSON line on rank 0)
     python bench.py --impl reference ...                          the reference's CPU algorithm (oracle port)
+    python bench.py ... --dump-outputs DIR                        also write the last timed step's results to DIR/*.npy
 
 `value`  : device-resident inputs, CUDA-event timed, max over ranks.
 `e2e`    : the same sweep through the public plugin call acquisition_function_withGradients(numpy) with
@@ -209,6 +210,24 @@ def workload_config(c, n_per_gpu):
             "l2": "256 MiB flush between steps; per-step K*/V scratch (GiBs) far exceeds the 126 MB L2"}
 
 
+DUMP_ROWS = 1 << 18      # 2^18 candidates x (acq + d-gradient + index) x 8 B = 25 MB at d = 10
+
+
+def dump_outputs(path, acq, grad_acq, topk):
+    """Write one step's results as float64 .npy files under `path`: the top-K records (value, global index, x) and, for a
+    fixed seeded sample of DUMP_ROWS candidates (all of them when there are fewer), acq, grad acq and the candidates'
+    row indices.  Two builds run with the same arguments can then be compared output for output."""
+    import torch
+    n = acq.shape[0]
+    idx = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    rows = torch.from_numpy(idx).to(acq.device)
+    arrays = {"acq": acq.reshape(-1)[rows], "grad_acq": grad_acq[rows], "candidate_index": idx, "topk": topk}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else a
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
+
+
 def bf16_peak():
     try:
         return float(json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json"))).get("bf16_tflops_sustained", 1400.0)), True
@@ -297,7 +316,6 @@ def quick_sweep(cname, N, dev, precision, steps=2, warmup=2, e2e=True, seed=0):
 def run_ours(args, cfg):
     import torch
     import torch.distributed as dist
-    import __graft_entry__ as ge
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -311,13 +329,12 @@ def run_ours(args, cfg):
         if os.environ.get("NCCL_DEBUG", "").upper() in ("VERSION", "INFO", "TRACE") and not os.environ.get("BOCF_KEEP_NCCL_DEBUG"):
             os.environ["NCCL_DEBUG_FILE"] = os.environ.get("NCCL_DEBUG_FILE", "/dev/stderr")
         dist.init_process_group("nccl", device_id=dev)
-    if rank == 0:
-        ge.build_library()
-    if world > 1:
-        dist.barrier()
     import bocf_b200
     from bocf_b200 import _lib, distributed as bd
     from tests.helpers import make_problem, product_model, product_utility
+    # the library comes from `python __graft_entry__.py` / build(): the benchmark compiles nothing and writes nothing
+    # into the tree, which may be read-only
+    _lib.load_library()
 
     c = dict(cfg)
     N = args.candidates or c["N"]
@@ -343,6 +360,7 @@ def run_ours(args, cfg):
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
 
     dbg = bool(os.environ.get("BOCF_BENCH_DEBUG"))
+    last = {}                                           # results of the latest step, for --dump-outputs
 
     def step_device():
         model.set_hyperparameters(0)
@@ -357,6 +375,7 @@ def run_ours(args, cfg):
             t3 = time.perf_counter()
             sys.stderr.write("    host: acq enqueue %.1f ms, topk enqueue %.1f ms, gather %.1f ms, drain %.1f ms\n"
                              % ((t1 - t0) * 1e3, (t2 - t1) * 1e3, 0.0, (t3 - t2) * 1e3))
+        last.update(acq=a, grad_acq=g, topk=out)
         return out
 
     def step_host():
@@ -412,6 +431,9 @@ def run_ours(args, cfg):
     ms_dev, _, launches, _ = timed(step_device, args.steps)
     value_step_ms = list(timed.last_step_ms)
     clocks = sampler.stop() if (rank == 0 and not os.environ.get("BOCF_BENCH_NO_SAMPLER")) else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, **last)
+    last.clear()
     # separate pass with per-kernel CUDA events (same steps, same data) for the roofline of the dominant kernel
     ms_prof, _, _, prof = timed(step_device, args.steps, profile=True)
     step_host()                                                     # warm the host path (pinned staging, allocator)
@@ -663,7 +685,13 @@ def main():
     ap.add_argument("--no-cfg5", action="store_true", help="skip the sharded configs[4] pass (N>=4)")
     ap.add_argument("--precision", default="auto", choices=["auto", "mixed", "fp64", "split3", "split4", "split5", "split6", "split54", "split43", "split53", "split44"],
                     help="arithmetic of the factor contractions (include/bocf_b200.h: enum bocf_precision)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     cfg = CONFIGS[args.config]
     # stdout must carry exactly ONE JSON line: libraries (NCCL's version banner, build logs, ...) that write to
     # fd 1 are diverted to stderr for the whole run; print() below goes to the saved real stdout.

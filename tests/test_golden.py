@@ -13,7 +13,7 @@ import pytest
 from tests.helpers import tol, Problem, oracle_model, oracle_acq, product_model, product_acq, rel_err
 
 GOLDEN = sorted(p for p in glob.glob(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "*.npz"))
-                if not os.path.basename(p).startswith(("lml_", "hmc_", "kg_")))   # lml_*: test_lml.py, hmc_*: test_hmc.py, kg_*: test_kg.py
+                if not os.path.basename(p).startswith(("lml_", "hmc_", "kg_", "grad_x_")))   # lml_*: test_lml.py, hmc_*: test_hmc.py, kg_*: test_kg.py, grad_x_*: test_oracle.py
 IDS = [os.path.basename(p)[:-4] for p in GOLDEN]
 
 
