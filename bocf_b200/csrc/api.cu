@@ -283,10 +283,6 @@ int bocf_model_create(bocf_model** out, int m, int d, int kernel, int device) {
   M->kinds.assign((size_t)m, kernel);
   M->device = device;
   M->precision = BOCF_PREC_AUTO;                                // library default
-  if (const char* env = std::getenv("BOCF_SCRATCH_GIB")) {     // per-chunk scratch limit (bocf_model_set_scratch_limit)
-    const double gib = std::atof(env);
-    if (gib >= 0.0625 && gib <= 160.0) M->scratch_limit = (uint64_t)(gib * 1073741824.0);
-  }
   if (const char* env = std::getenv("BOCF_PRECISION")) {      // fp64 | auto | mixed | split3 .. split6 | split<s1><s2>
     const std::string v(env);
     if (v == "auto") M->precision = BOCF_PREC_AUTO;
@@ -756,13 +752,8 @@ int bocf_acq_eval(bocf_model* M, int variant, int composite, const double* Xc, i
 
   // Variants with gradients on the tensor-core contraction path: the fused gradient sweep (posterior.cu) -- the
   // per-output mean / variance gradients are never materialised (MC variants; the analytic ones up to 16 outputs, whose
-  // weights live in registers).  BOCF_FUSED_GRAD=0 keeps the unfused sequence.
-  static int fused_on = -1;
-  if (fused_on < 0) {
-    const char* env = std::getenv("BOCF_FUSED_GRAD");
-    fused_on = (env && std::atoi(env) == 0) ? 0 : 1;
-  }
-  const bool fused = fused_on && grad && M->S > 0 &&
+  // weights live in registers).
+  const bool fused = grad && M->S > 0 &&
                      (variant == BOCF_ACQ_EI_CF || variant == BOCF_ACQ_MEAN_UTILITY ||
                       ((variant == BOCF_ACQ_MA_EI || variant == BOCF_ACQ_MA_PI) && M->m <= 16));
   for (int64_t off = 0; off < N; off += Nc) {

@@ -684,8 +684,7 @@ int launch_gram(bocf_model* M, OutRun grp, cudaStream_t st) {
 
 // Two output groups on two streams when there are enough matrices for it to pay (see GroupStreams, model.h).
 int for_each_output_group(bocf_model* M, cudaStream_t st, int (*f)(bocf_model*, OutRun, cudaStream_t, void*), void* ctx) {
-  static const bool off = std::getenv("BOCF_NO_GROUPS") != nullptr;
-  if (M->m < 4 || M->H * M->m < 8 || M->nb < 3 || off) return f(M, OutRun{0, M->m}, st, ctx);
+  if (M->m < 4 || M->H * M->m < 8 || M->nb < 3) return f(M, OutRun{0, M->m}, st, ctx);
   GroupStreams& gs = M->gs;
   if (!gs.side) {
     BOCF_CUDA_OK(cudaStreamCreateWithFlags(&gs.side, cudaStreamNonBlocking));

@@ -17,27 +17,6 @@
 // results, far inside the 1e-6 / 1e-9 parity bars.
 #pragma once
 #include "model.h"
-// Compile-time switches of the K* arithmetic (defaults = fastest measured, profiles/r1_split_experiments.md section 10):
-//   KV_EXPSEL   1: exp clamps at -700 without the final flush-to-zero select      KV_SQRTBIAS 1: sqrt biased by 1e-300, no select
-//   KV_CONST    1: sqrt(5), 5/3 ... from constant memory instead of literals       KV_LB: min CTAs/SM in kstar's launch bounds
-#ifndef KV_EXPSEL
-#define KV_EXPSEL 1
-#endif
-#ifndef KV_SQRTBIAS
-#define KV_SQRTBIAS 1
-#endif
-#ifndef KV_CONST
-#define KV_CONST 1
-#endif
-#ifndef KV_LB
-#define KV_LB 1
-#endif
-#ifndef KV_SQRTSHORT
-#define KV_SQRTSHORT 1
-#endif
-#ifndef KV_EXPTAB
-#define KV_EXPTAB 1
-#endif
 
 namespace bocf {
 
@@ -87,12 +66,7 @@ __device__ __forceinline__ double exp_nonpos(double x) {
   p = fma(p, r, 1.0);
   p = fma(p, r, 1.0);
   const int k = __double2loint(sh);
-#if KV_EXPSEL
   return __hiloint2double(__double2hiint(p) + (k << 20), __double2loint(p));
-#else
-  const double scaled = __hiloint2double(__double2hiint(p) + (k << 20), __double2loint(p));
-  return (x < EXPC[15]) ? 0.0 : scaled;
-#endif
 }
 
 // Table variant for the K* kernel: x = (128 k + j) ln2/128 + r, |r| <= ln2/256, exp(x) = 2^k * 2^(j/128) * p(r) with a
@@ -162,36 +136,18 @@ __device__ __forceinline__ double clamp_q(double q, bool& nz) {
 // sqrt(a) for a >= 0 (finite).  libdevice's rsqrt(double) wraps the hardware seed (MUFU.RSQ64H, ~22 bits) in a range check
 // with an out-of-line slow path; that branch (BSSY / CALL / BSYNC per evaluation) keeps ptxas from interleaving the
 // independent distance -> kernel chains of an unrolled trip.  Here the seed is taken directly (rsqrt.approx.ftz.f64) and
-// refined branch-free: y <- y (1 + e/2 + 3 e^2/8) with e = 1 - a y^2 (cubic, error ~e^3 ~ 1e-20), then one Newton step on
-// s = a y.  The argument is biased by 1e-300 (a no-op for a > 1e-284) so the seed stays finite at a == 0: sqrt(0) comes
+// refined branch-free: y <- y (1 + e/2 + 3 e^2/8) with e = 1 - a y^2 (cubic, error ~e^3 ~ 1e-20), and the root is
+// a y.  The argument is biased by 1e-300 (a no-op for a > 1e-284) so the seed stays finite at a == 0: sqrt(0) comes
 // out as 1e-150 instead of 0, which no kernel value can see (1 + sqrt5 * 1e-150 == 1) -- one add instead of a compare and
 // two selects.
 __device__ __forceinline__ double sqrt_nonneg(double a0) {
-#if KV_SQRTBIAS
   const double a = a0 + KERC[4];
-#else
-  const double a = a0;
-#endif
   double y;
   asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(a));
   const double e = fma(-a * y, y, 1.0);
   const double p = fma(0.375, e, 0.5);
   y = fma(y * e, p, y);
-  double s = a * y;
-#if KV_SQRTBIAS && KV_SQRTSHORT
-  const double r = 0.0;
-#else
-  const double r = fma(-s, s, a);
-#endif
-#if KV_SQRTBIAS && KV_SQRTSHORT
-  (void)r;
-  return s;                        // y carries ~1e-20 after the cubic step: a*y is within 1.5 ulp of sqrt(a)
-#elif KV_SQRTBIAS
-  return fma(r, 0.5 * y, s);
-#else
-  s = fma(r, 0.5 * y, s);
-  return (a > 1e-300) ? s : 0.0;
-#endif
+  return a * y;                    // y carries ~1e-20 after the cubic step: a*y is within 1.5 ulp of sqrt(a)
 }
 
 #define BOCF_EXP(x) (variance * exp_nonpos(x))
@@ -208,19 +164,11 @@ __device__ __forceinline__ void kern_eval(double r2, double variance, double& k,
   } else if (KIND == BOCF_KERN_MATERN52) {
     // stationary.py:529-533
     const double r = sqrt_nonneg(r2);
-#if KV_CONST
     const double t = KERC[0] * r;               // sqrt(5) r
     const double e = BOCF_EXP(-t);
     const double lin = 1.0 + t;
     k = fma(KERC[1], r2, lin) * e;
     if (GRAD) g = (r2 != 0.0) ? KERC[2] * (lin * e) : 0.0;
-#else
-    const double s5 = 2.23606797749978969641;   // sqrt(5)
-    const double e = BOCF_EXP(-s5 * r);
-    const double lin = 1.0 + s5 * r;
-    k = (lin + 5.0 / 3.0 * r2) * e;
-    if (GRAD) g = (r2 != 0.0) ? (-5.0 / 3.0) * (lin * e) : 0.0;
-#endif
   } else {
     // Matern32, stationary.py:440-444
     const double r = sqrt_nonneg(r2);

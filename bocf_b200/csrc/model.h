@@ -180,9 +180,10 @@ int split_linv_absmax(bocf_model* M, double* out_host, cudaStream_t st);
 uint64_t split_chunk_bytes_per_candidate(const bocf_model* M, bool grad, int64_t Nc = 0);
 void split_carve_chunk(const bocf_model* M, void* base, int64_t Nc, bool grad, ChunkBuffers* out);
 int launch_split_var(bocf_model* M, int h, int64_t Nvalid, const ChunkBuffers& cb, bool need_dvar, cudaStream_t st);
-int launch_split_dvar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, const ChunkBuffers& cb, cudaStream_t st);
-// second contraction with the fused acquisition-gradient epilogue (weights cb.wa / cb.wb, alpha of the model)
-int launch_split_dacq(bocf_model* M, int h, const double* Xc, int64_t Nvalid, const ChunkBuffers& cb, cudaStream_t st);
+// second contraction: per-output variance gradients, or with fused_acq the acquisition-gradient epilogue (weights
+// cb.wa / cb.wb, alpha of the model)
+int launch_split_dvar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, const ChunkBuffers& cb, bool fused_acq,
+                      cudaStream_t st);
 int split_debug_gemm(const double* A, const double* B, int R, int N, int K, int sch, int tri, double* out, cudaStream_t st);
 
 // ---- kg.cu --------------------------------------------------------------------------------------

@@ -53,7 +53,7 @@ struct SplitOut {
 //       (api.cu) folds the mean-gradient contraction into the second contraction's epilogue, which saves the d + 2
 //       fp64 operations per (candidate, training point) the mean gradient costs here.
 template <int KIND, int DP, int GRAD, int SPL>
-__global__ void __launch_bounds__(128, KV_LB) kstar_kernel(const double* __restrict__ Xc, int64_t Nvalid, int64_t Nc, int d,
+__global__ void __launch_bounds__(128, 1) kstar_kernel(const double* __restrict__ Xc, int64_t Nvalid, int64_t Nc, int d,
                                                     int n, int n16, int n_pad, int m, int h,
                                                     const OutHyp* __restrict__ hyp, const double* __restrict__ XsAll,
                                                     const double* __restrict__ xsqAll,
@@ -73,17 +73,14 @@ __global__ void __launch_bounds__(128, KV_LB) kstar_kernel(const double* __restr
   __shared__ double sexp[EXP_TAB_N];
   const int tid = threadIdx.x;
   // visible after the first __syncthreads of the tile loop; the output's signal variance rides in the table entries
-  if (KV_EXPTAB) exp_table_fill(sexp, tid, hyp[h * m + j0 + blockIdx.y].variance);
+  exp_table_fill(sexp, tid, hyp[h * m + j0 + blockIdx.y].variance);
   const int j = j0 + blockIdx.y;                 // this launch covers one run of outputs that share the kernel family
   const int hj = h * m + j;
   const int64_t i = (int64_t)blockIdx.x * 128 + tid;
   const OutHyp& hp = hyp[hj];
-  const double variance = hp.variance;
 
-  // FAST arithmetic (kernfn.cuh): everything the kernel family multiplies the squared distance by is folded into the
-  // operands of the distance itself:  q = SCALE r2 = SCALE (|x|^2 + |X_b|^2) + sum_q (-2 SCALE x_q) X_bq
-  constexpr bool FAST = (KV_EXPTAB != 0);
-  constexpr double QS = FAST ? KFast<KIND>::SCALE : 1.0;
+  // everything the kernel family multiplies the squared distance by (kernfn.cuh: KFast) is folded into the operands of
+  // the distance itself:  q = SCALE r2 = SCALE (|x|^2 + |X_b|^2) + sum_q (-2 SCALE x_q) X_bq
   double xs[DP], xm2[DP];
   double xsq_i = 0.0;
 #pragma unroll
@@ -91,10 +88,10 @@ __global__ void __launch_bounds__(128, KV_LB) kstar_kernel(const double* __restr
     double v = 0.0;
     if (q < d && i < Nvalid) v = Xc[i * d + q] / hp.ls[q];
     xs[q] = v;
-    xm2[q] = (-2.0 * QS) * v;
+    xm2[q] = (-2.0 * KFast<KIND>::SCALE) * v;
     xsq_i += v * v;
   }
-  xsq_i *= QS;
+  xsq_i *= KFast<KIND>::SCALE;
   double mu = 0.0, wsum = 0.0;
   double gm[DP];       // sum_b w_b Xs_bq ;  dmean_q = (xs_q * sum_b w_b - gm_q) / l_q
 #pragma unroll
@@ -104,7 +101,7 @@ __global__ void __launch_bounds__(128, KV_LB) kstar_kernel(const double* __restr
   const double* xsq = xsqAll + (int64_t)hj * n_pad;
   const double* alpha = alphaAll + (int64_t)hj * n_pad;
   constexpr bool SPLIT = SPL > 0;
-  constexpr bool GFOLD = FAST && SPLIT && GRAD == 2;
+  constexpr bool GFOLD = SPLIT && GRAD == 2;
   double* Kout = SPLIT ? nullptr : KsT + (int64_t)j * n16 * Nc;
   double* Gout = GRAD ? GsT + (int64_t)j * n16 * Nc : nullptr;
   // split mode: digit planes of this block's 128 candidates (row = tid) for output j
@@ -127,10 +124,10 @@ __global__ void __launch_bounds__(128, KV_LB) kstar_kernel(const double* __restr
     }
     {
       int b = b0 + tid;
-      sxsq[tid] = (b < n) ? QS * xsq[b] : 0.0;
+      sxsq[tid] = (b < n) ? KFast<KIND>::SCALE * xsq[b] : 0.0;
       salpha[tid] = (b < n) ? alpha[b] : 0.0;
       // column scale of the second contraction times the 256 its epilogue's merged Horner leaves out (split_gemm.cu)
-      // (and, on the FAST path, the constant factor of (dK/dr)/r that kern_eval_fast leaves out)
+      // (and, when GFOLD, the constant factor of (dK/dr)/r that kern_eval_fast leaves out)
       if (SPL > 0) sgcs[tid] = (b < n) ? (GFOLD ? 256.0 * KFast<KIND>::GFAC : 256.0) * so.gcs[(size_t)hj * so.gcs_ld + b] : 0.0;
     }
     __syncthreads();
@@ -158,7 +155,7 @@ __global__ void __launch_bounds__(128, KV_LB) kstar_kernel(const double* __restr
                 r2b = fma(d1, d1, r2b);
               }
             }
-            r2 = QS * (r2a + r2b);
+            r2 = KFast<KIND>::SCALE * (r2a + r2b);
           } else {
             // two chains (half the dependent-DFMA depth), seeded with the two squared norms: d DFMA + 1 DADD
             double dot0 = xsq_i, dot1 = sxsq[bb];
@@ -169,16 +166,11 @@ __global__ void __launch_bounds__(128, KV_LB) kstar_kernel(const double* __restr
             }
             r2 = dot0 + dot1;
           }
-          if (FAST) {
-            // clip at 0 (stationary.py:153) and the cap that replaces exp's clamp, on the integer pipe
-            bool nz;
-            const double qc = clamp_q<KIND>(r2, nz);
-            kern_eval_fast<KIND, (GRAD != 0)>(qc, nz, kv, gv, sexp);
-            if (GRAD && !GFOLD) gv *= KFast<KIND>::GFAC;
-          } else {
-            if (KIND != BOCF_KERN_SE) r2 = fmax(r2, 0.0);
-            kern_eval<KIND, (GRAD != 0)>(r2, variance, kv, gv);
-          }
+          // clip at 0 (stationary.py:153) and the cap that replaces exp's clamp, on the integer pipe
+          bool nz;
+          const double qc = clamp_q<KIND>(r2, nz);
+          kern_eval_fast<KIND, (GRAD != 0)>(qc, nz, kv, gv, sexp);
+          if (GRAD && !GFOLD) gv *= KFast<KIND>::GFAC;
           // padded points b >= n need no mask: their alpha, column scale and factor rows / columns are zero, so whatever
           // finite K*, G* they produce is multiplied by an exact zero downstream (mean, both contractions, epilogues)
           const double a = salpha[bb];
@@ -637,7 +629,7 @@ int launch_fused_grad_chunk(bocf_model* M, int h, const double* Xc, int64_t Nval
   P.wa = cb.wa;
   P.wb = cb.wb;
   if (int rc = launch_acq_chunk(P, cb, Nvalid, acq, nullptr, st)) return rc;
-  if (int rc = launch_split_dacq(M, h, Xc, Nvalid, cb, st)) return rc;
+  if (int rc = launch_split_dvar(M, h, Xc, Nvalid, cb, true, st)) return rc;
   {
     ProfScope ps("finalize_kernel", st);
     if (Nvalid <= 128)
@@ -673,7 +665,7 @@ int launch_posterior_chunk(bocf_model* M, int h, const double* Xc, int64_t Nvali
     // tcgen05 kind::i8 digit-plane contractions (split_gemm.cu); same partial-sum layout, same finalize
     if (int rc2 = launch_split_var(M, h, Nvalid, cb, need_dvar, st)) return rc2;
     if (need_dvar)
-      if (int rc2 = launch_split_dvar(M, h, Xc, Nvalid, cb, st)) return rc2;
+      if (int rc2 = launch_split_dvar(M, h, Xc, Nvalid, cb, false, st)) return rc2;
   } else {
   {
     ProfScope ps("var_gemm_kernel", st);

@@ -37,7 +37,6 @@
 //            The sums live in registers across all column tiles of a work unit (see NP below).
 // Triangular structure of Linv is exploited per column tile: K chunks (64) for the loads, K steps (32) for the MMAs.
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -120,15 +119,6 @@ struct Cfg {
   static_assert(EPI_WARPS % 4 == 0 && (NT / 8) % PART_SPLIT == 0, "column groups must divide evenly over the warps");
 };
 
-// Knock-out build (-DBOCF_KNOCKOUT, never the shipped library): BOCF_SPLIT_EXP is a bit mask -- 1 skips the MMAs,
-// 2 the bulk loads, 4 the epilogue work, 8 only the V-digit stores, 16 only the epilogue arithmetic (TMEM loads stay).
-// Results are invalid; only time / energy are read (scripts/dev_knockout.sh).
-#ifdef BOCF_KNOCKOUT
-#define BOCF_KO(x) ((P.exp & (x)) != 0)
-#else
-#define BOCF_KO(x) false
-#endif
-
 // EPI_DACQ: the second contraction with the fused acquisition-gradient epilogue -- instead of T = Wt G* it contracts
 //   u_b = G*_b (WA_j alpha_b - 2 WB_j Wt_b)      (WA, WB: per-candidate weights from the MC pass, acq.cu)
 // so that sum_j (xs_j sum_b u_b - sum_b u_b Xs_b) / l_j = sum_j WA_j dmu_j + WB_j dvar_j = grad acq  (uEI_noiseless.py:163-166).
@@ -163,8 +153,6 @@ struct GemmParams {
   const OutHyp* hyp;
   int d, n16, n_pad;
   int np;                  // parts per candidate tile
-  int l2_keep_a;           // 1: A planes loaded with an L2 evict_last policy (BOCF_SPLIT_L2KEEP)
-  int exp;                 // knock-out builds only
 };
 
 // Work decomposition.  A UNIT is (output j, candidate tile rt, part p of NP): the column tiles ct = p, p+NP, ... of one
@@ -173,18 +161,6 @@ struct GemmParams {
 // instead of one per column tile.  NP = 1 (a CTA owns the whole row of column tiles of its candidate tile) measured
 // best on B200: 354 vs 371 (NP = 2) vs 390 ms (NP = 4) per 1M-candidate step at cfg 3 -- fewer partial sums, and the
 // tile's digit planes are re-read by one SM back to back.  More parts only pay when there are fewer units than SMs.
-constexpr int NP_DEFAULT = 1;   // parts per candidate tile (BOCF_SPLIT_NP overrides: 1, 2, 4 or 8)
-inline int parts_env() {        // 0: no override
-  static int np = -1;
-  if (np < 0) {
-    np = 0;
-    if (const char* env = std::getenv("BOCF_SPLIT_NP")) {
-      const int v = std::atoi(env);
-      if (v == 1 || v == 2 || v == 4 || v == 8) np = v;
-    }
-  }
-  return np;
-}
 // Two reasons to give a candidate tile to more than one CTA:
 //  * small batches (the L-BFGS rounds of the acquisition optimiser: tens of candidates = one candidate tile per output)
 //    have fewer units than SMs;
@@ -193,8 +169,7 @@ inline int parts_env() {        // 0: no override
 //    148 = 382 MB at n = 4000 -- there the re-streaming went to HBM and both contractions ran HBM-bound (cfg 5: 0.99 /
 //    0.81 s per 200k candidates with one part, 0.59 / 0.54 s with four CTAs sharing each tile).
 inline int parts_for(int units_at_np1, int sms, int64_t a_tile_bytes, int64_t l2_bytes) {
-  if (parts_env()) return parts_env();
-  int np = NP_DEFAULT;
+  int np = 1;
   if (units_at_np1 * 4 <= sms) np = 4;            // 8 parts measured no faster at 17 candidates: a small batch still
   else if (units_at_np1 * 2 <= sms) np = 2;       // streams every factor plane (148 MB at cfg 3), that is its floor
   const int64_t budget = l2_bytes * 4 / 5;
@@ -402,7 +377,6 @@ __global__ void __launch_bounds__(Cfg<SCH, DP>::NTHREADS, 1) split_gemm_kernel(c
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      const uint64_t pol_keep = tc::l2_policy_evict_last();
       TileWalk<NT> walk;
       walk.start(P);
       TileInfo ti;
@@ -418,18 +392,8 @@ __global__ void __launch_bounds__(Cfg<SCH, DP>::NTHREADS, 1) split_gemm_kernel(c
         }
         for (int kc = ti.kb; kc < ti.ke; ++kc) {
           tc::mbar_wait(&empty[stage], phase ^ 1u);
-          if (BOCF_KO(2)) {
-            tc::mbar_arrive(&full[stage]);
-            if (++stage == C::STAGES) {
-              stage = 0;
-              phase ^= 1u;
-            }
-            continue;
-          }
           tc::mbar_arrive_expect_tx(&full[stage], C::STAGE);
-          // the unit's A tile is re-streamed once per column tile: ask L2 to keep it (P.l2_keep_a)
-          if (P.l2_keep_a) tc::bulk_g2s_hint(sA + stage * C::A_STAGE, gA + (size_t)kc * C::A_STAGE, C::A_STAGE, &full[stage], pol_keep);
-          else tc::bulk_g2s(sA + stage * C::A_STAGE, gA + (size_t)kc * C::A_STAGE, C::A_STAGE, &full[stage]);
+          tc::bulk_g2s(sA + stage * C::A_STAGE, gA + (size_t)kc * C::A_STAGE, C::A_STAGE, &full[stage]);
           tc::bulk_g2s(sB + stage * C::B_STAGE, gB + (size_t)kc * C::B_STAGE, C::B_STAGE, &full[stage]);
           if (++stage == C::STAGES) {
             stage = 0;
@@ -464,7 +428,6 @@ __global__ void __launch_bounds__(Cfg<SCH, DP>::NTHREADS, 1) split_gemm_kernel(c
         for (int ks = 0; ks < KC / 32; ++ks) {
           const int kstep = kc * (KC / 32) + ks;            // K steps wholly outside the triangle multiply zeros: skip
           if (kstep < ti.sb || kstep >= ti.se) continue;
-          if (BOCF_KO(1)) continue;
           if (first) {
             if (tc::elect_one()) issue_kstep<C, true>(a_lo + ks * 2, b_lo + ks * 2, d_tmem);
           } else {
@@ -594,39 +557,23 @@ __global__ void __launch_bounds__(Cfg<SCH, DP>::NTHREADS, 1) split_gemm_kernel(c
       // register buffers), so the TMEM round trip overlaps the fp64 work.  The gradient epilogues, whose 2 d + 2
       // accumulators leave fewer registers, do the same with 4-column groups (two buffers of NL x 4 words = the one
       // buffer of NL x 8 they had: the exposed TMEM latency was 12 % of their samples in ncu).
-      constexpr bool PREF = true;
-      uint32_t c[PREF ? 2 : 1][NL][CGW];
-      if (PREF) {
+      uint32_t c[2][NL][CGW];
 #pragma unroll
-        for (int lb = 0; lb < NL; ++lb) tc::tmem_ldw<CGW>(taddr + (uint32_t)(lb * NT + hw * CGW), c[0][lb]);
-      }
+      for (int lb = 0; lb < NL; ++lb) tc::tmem_ldw<CGW>(taddr + (uint32_t)(lb * NT + hw * CGW), c[0][lb]);
 #pragma unroll
       for (int gi = 0; gi < NGW; ++gi) {
-        if (BOCF_KO(4)) {
-          if (PREF) tc::tmem_ld_wait();
-          break;
-        }
         const int cg = hw + gi * PART_SPLIT;
-        constexpr int dummy = 0;
-        (void)dummy;
-        if (PREF) {
-          tc::tmem_ld_wait();
-          if (gi + 1 < NGW) {
+        tc::tmem_ld_wait();
+        if (gi + 1 < NGW) {
 #pragma unroll
-            for (int lb = 0; lb < NL; ++lb)
-              tc::tmem_ldw<CGW>(taddr + (uint32_t)(lb * NT + (cg + PART_SPLIT) * CGW), c[(gi + 1) & 1][lb]);
-          }
-        } else {
-#pragma unroll
-          for (int lb = 0; lb < NL; ++lb) tc::tmem_ldw<CGW>(taddr + (uint32_t)(lb * NT + cg * CGW), c[0][lb]);
-          tc::tmem_ld_wait();
+          for (int lb = 0; lb < NL; ++lb)
+            tc::tmem_ldw<CGW>(taddr + (uint32_t)(lb * NT + (cg + PART_SPLIT) * CGW), c[(gi + 1) & 1][lb]);
         }
-        const uint32_t (&cc)[NL][CGW] = c[PREF ? (gi & 1) : 0];
+        const uint32_t (&cc)[NL][CGW] = c[gi & 1];
         uint32_t vec[S2][CGW / 4];
         unsigned long long dgv[CGW];
 #pragma unroll
         for (int e = 0; e < CGW; ++e) {
-          if (BOCF_KO(16)) break;
           if (EPI == EPI_RAW) {
             const double v = levels_to_f64<NL, CGW>(cc, e) * cs_t[cg * CGW + e].x;
             const int col = col0 + cg * CGW + e;
@@ -659,16 +606,7 @@ __global__ void __launch_bounds__(Cfg<SCH, DP>::NTHREADS, 1) split_gemm_kernel(c
             }
           }
         }
-        if (BOCF_KO(16)) {                                       // keep the loads alive, skip the arithmetic
-          uint32_t x = 0;
-#pragma unroll
-          for (int lb = 0; lb < NL; ++lb)
-#pragma unroll
-            for (int e = 0; e < CGW; ++e) x ^= cc[lb][e];
-          if (x == 0x9e3779b9u) sumsq += 1.0;
-          continue;
-        }
-        if (EPI == EPI_VAR && P.A2 != nullptr && !BOCF_KO(8)) {
+        if (EPI == EPI_VAR && P.A2 != nullptr) {
 #pragma unroll
           for (int w = 0; w < CGW / 4; ++w) {                    // byte transpose: digit t of 4 columns -> one word
             const unsigned long long four[4] = {dgv[4 * w], dgv[4 * w + 1], dgv[4 * w + 2], dgv[4 * w + 3]};
@@ -860,41 +798,25 @@ static int launch_var(int sch, int s2, const GemmParams& P, cudaStream_t st) {
   }
   return bad_scheme();
 }
-template <int DP>
-static int launch_dvar_d(int sch, const GemmParams& P, cudaStream_t st) {
+// second contraction (EPI_DVAR or EPI_DACQ) with scheme `sch` for d input dimensions
+template <int EPI, int DP>
+static int launch_grad_d(int sch, const GemmParams& P, cudaStream_t st) {
   switch (sch) {
-    case 331: return launch_k<P331, EPI_DVAR, DP, 3>(P, st);
-    case 442: return launch_k<P442, EPI_DVAR, DP, 4>(P, st);
-    case 554: return launch_k<P554, EPI_DVAR, DP, 5>(P, st);
-    case 665: return launch_k<P665, EPI_DVAR, DP, 6>(P, st);
+    case 331: return launch_k<P331, EPI, DP, 3>(P, st);
+    case 442: return launch_k<P442, EPI, DP, 4>(P, st);
+    case 554: return launch_k<P554, EPI, DP, 5>(P, st);
+    case 665: return launch_k<P665, EPI, DP, 6>(P, st);
   }
   return bad_scheme();
 }
-template <int DP>
-static int launch_dacq_d(int sch, const GemmParams& P, cudaStream_t st) {
-  switch (sch) {
-    case 331: return launch_k<P331, EPI_DACQ, DP, 3>(P, st);
-    case 442: return launch_k<P442, EPI_DACQ, DP, 4>(P, st);
-    case 554: return launch_k<P554, EPI_DACQ, DP, 5>(P, st);
-    case 665: return launch_k<P665, EPI_DACQ, DP, 6>(P, st);
-  }
-  return bad_scheme();
-}
-static int launch_dacq(int sch, int d, const GemmParams& P, cudaStream_t st) {
-  if (d <= 4) return launch_dacq_d<4>(sch, P, st);
-  if (d <= 6) return launch_dacq_d<6>(sch, P, st);
-  if (d <= 8) return launch_dacq_d<8>(sch, P, st);
-  if (d <= 10) return launch_dacq_d<10>(sch, P, st);
-  if (d <= 12) return launch_dacq_d<12>(sch, P, st);
-  return launch_dacq_d<16>(sch, P, st);
-}
-static int launch_dvar(int sch, int d, const GemmParams& P, cudaStream_t st) {
-  if (d <= 4) return launch_dvar_d<4>(sch, P, st);
-  if (d <= 6) return launch_dvar_d<6>(sch, P, st);
-  if (d <= 8) return launch_dvar_d<8>(sch, P, st);
-  if (d <= 10) return launch_dvar_d<10>(sch, P, st);
-  if (d <= 12) return launch_dvar_d<12>(sch, P, st);
-  return launch_dvar_d<16>(sch, P, st);
+template <int EPI>
+static int launch_grad(int sch, int d, const GemmParams& P, cudaStream_t st) {
+  if (d <= 4) return launch_grad_d<EPI, 4>(sch, P, st);
+  if (d <= 6) return launch_grad_d<EPI, 6>(sch, P, st);
+  if (d <= 8) return launch_grad_d<EPI, 8>(sch, P, st);
+  if (d <= 10) return launch_grad_d<EPI, 10>(sch, P, st);
+  if (d <= 12) return launch_grad_d<EPI, 12>(sch, P, st);
+  return launch_grad_d<EPI, 16>(sch, P, st);
 }
 
 }  // namespace sg
@@ -1082,13 +1004,6 @@ static sg::GemmParams base_params(const bocf_model* M, int h, const ChunkBuffers
   P.n_pad = M->n_pad;
   P.hyp = M->hyp;
   P.np = split_parts(M, cb.Nc);
-  static int keep = -1;
-  if (keep < 0) {
-    const char* env = std::getenv("BOCF_SPLIT_L2KEEP");
-    keep = (env && std::atoi(env) != 0) ? 1 : 0;
-  }
-  P.l2_keep_a = keep;
-  if (const char* env = std::getenv("BOCF_SPLIT_EXP")) P.exp = std::atoi(env);
   return P;
 }
 
@@ -1108,7 +1023,8 @@ int launch_split_var(bocf_model* M, int h, int64_t Nvalid, const ChunkBuffers& c
   return sg::launch_var(M->sch1, M->S2, P, st);
 }
 
-int launch_split_dvar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, const ChunkBuffers& cb, cudaStream_t st) {
+int launch_split_dvar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, const ChunkBuffers& cb, bool fused_acq,
+                      cudaStream_t st) {
   sg::GemmParams P = base_params(M, h, cb, Nvalid);
   P.A = cb.A2;
   P.B = M->B2;
@@ -1119,38 +1035,18 @@ int launch_split_dvar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, co
   P.part_s0 = cb.part_s0;
   P.GsT = cb.GsT;
   P.Xc = Xc;
-  P.Nvalid = Nvalid;
   P.Xs = M->Xs;
+  if (fused_acq) {
+    P.alpha = M->alpha;
+    P.wa = cb.wa;
+    P.wb = cb.wb;
+  }
   if (M->nct2 < P.np) {
     BOCF_CUDA_OK(cudaMemsetAsync(cb.part_dvar, 0, sizeof(double) * M->m * split_partials_dvar(M, cb.Nc) * cb.Nc * M->d, st));
     BOCF_CUDA_OK(cudaMemsetAsync(cb.part_s0, 0, sizeof(double) * M->m * split_partials_dvar(M, cb.Nc) * cb.Nc, st));
   }
   ProfScope ps("split_dvar_kernel", st);
-  return sg::launch_dvar(M->sch2, M->d, P, st);
-}
-
-int launch_split_dacq(bocf_model* M, int h, const double* Xc, int64_t Nvalid, const ChunkBuffers& cb, cudaStream_t st) {
-  sg::GemmParams P = base_params(M, h, cb, Nvalid);
-  P.A = cb.A2;
-  P.B = M->B2;
-  P.cs = M->cs2;
-  P.nct = M->nct2;
-  P.tri = sg::TRI_K_GE_N;
-  P.part_dvar = cb.part_dvar;
-  P.part_s0 = cb.part_s0;
-  P.GsT = cb.GsT;
-  P.Xc = Xc;
-  P.Nvalid = Nvalid;
-  P.Xs = M->Xs;
-  P.alpha = M->alpha;
-  P.wa = cb.wa;
-  P.wb = cb.wb;
-  if (M->nct2 < P.np) {
-    BOCF_CUDA_OK(cudaMemsetAsync(cb.part_dvar, 0, sizeof(double) * M->m * split_partials_dvar(M, cb.Nc) * cb.Nc * M->d, st));
-    BOCF_CUDA_OK(cudaMemsetAsync(cb.part_s0, 0, sizeof(double) * M->m * split_partials_dvar(M, cb.Nc) * cb.Nc, st));
-  }
-  ProfScope ps("split_dvar_kernel", st);
-  return sg::launch_dacq(M->sch2, M->d, P, st);
+  return fused_acq ? sg::launch_grad<sg::EPI_DACQ>(M->sch2, M->d, P, st) : sg::launch_grad<sg::EPI_DVAR>(M->sch2, M->d, P, st);
 }
 
 // Test entry: out (R x N) = A (R x K) * B (N x K)^T through the digit-plane machinery.  All pointers [dev] fp64 row-major.
@@ -1191,7 +1087,7 @@ int split_debug_gemm(const double* A, const double* B, int R, int N, int K, int 
     P.cs = cs;
     P.m = 1;
     P.h = 0;
-    P.np = sg::parts_env() ? sg::parts_env() : sg::NP_DEFAULT;
+    P.np = 1;
     P.RT = RT;
     P.RTv = RT;
     P.nct = nct;

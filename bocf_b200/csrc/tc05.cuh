@@ -61,27 +61,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
                : "memory");
 }
 
-// Same with an L2 eviction-priority policy (createpolicy): evict_last keeps a tile that is re-streamed many times resident
-// against the streaming traffic of the epilogues.
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;\n" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;\n" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void bulk_g2s_hint(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar,
-                                              uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;\n" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
-      : "memory");
-}
-
 // L2 prefetch of a contiguous global range (multiple of 16 bytes), fire and forget.
 __device__ __forceinline__ void prefetch_l2(const void* gmem_src, uint32_t bytes) {
   asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;\n" ::"l"(gmem_src), "r"(bytes) : "memory");

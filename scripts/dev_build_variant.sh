@@ -1,6 +1,6 @@
 #!/bin/bash
 # Build a variant of the library next to the default one for A/B timing (scripts/dev_variant_bench.sh picks it up through
-# BOCF_LIB_PATH):   scripts/dev_build_variant.sh lb3 posterior.cu -DKV_LB=3   ->  bocf_b200/csrc/libbocf_lb3.so
+# BOCF_LIB_PATH):   scripts/dev_build_variant.sh rr128 posterior.cu -maxrregcount=128   ->  bocf_b200/csrc/libbocf_rr128.so
 # The other objects are the default build's (run `python __graft_entry__.py` first).  Variant .so files are git-ignored.
 set -e
 name=$1; src=$2; shift 2

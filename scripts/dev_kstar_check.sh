@@ -8,10 +8,3 @@ timeout 300 python bench.py --steps 3 --warmup 3 --no-cpu-baseline --no-mixed --
 echo "bench rc=$?"
 python -c "
 import json; d=json.load(open('gpurun_out/bench_kstar.json')); print(round(d['value']), round(d['ms_per_step'],1), {k:round(v/3,1) for k,v in d['roofline']['kernel_ms'].items()}, d['clocks']['sm_mhz'])"
-# optional: the same bench with posterior.cu built at -DKV_LB=3 (libbocf_lb3.so, when present)
-if [ -f bocf_b200/csrc/libbocf_lb3.so ]; then
-  BOCF_LIB_PATH=$PWD/bocf_b200/csrc/libbocf_lb3.so timeout 300 python bench.py --steps 3 --warmup 3 --no-cpu-baseline --no-mixed --no-extras > gpurun_out/bench_kstar_lb3.json 2> gpurun_out/bench_kstar_lb3.err
-  echo "lb3 bench rc=$?"
-  python -c "
-import json; d=json.load(open('gpurun_out/bench_kstar_lb3.json')); print(round(d['value']), round(d['ms_per_step'],1), {k:round(v/3,1) for k,v in d['roofline']['kernel_ms'].items()}, d['clocks']['sm_mhz'])"
-fi

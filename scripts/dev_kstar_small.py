@@ -1,4 +1,5 @@
-"""K* latency at small batches: thread-per-candidate kernel vs the 16-threads-per-candidate variant (BOCF_KSTAR_SMALL_MAX)."""
+"""K* latency at small batches (kstar_kernel splits the training points over blocks for chunks up to 1024 candidates):
+wall time per call and per-kernel times, K* alone and with the full posterior."""
 import os, sys, time
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -19,5 +20,5 @@ for N in (17, 256, 1024):
         torch.cuda.synchronize()
         wall = (time.perf_counter() - t0) / 50
         prof = _lib.profile_report(); _lib.profile_enable(False)
-        print("small_max=%s N=%4d %-15s wall %7.1f us/call  kernels(us): %s" % (os.environ.get("BOCF_KSTAR_SMALL_MAX", "default"), N, what, 1e6 * wall,
+        print("N=%4d %-15s wall %7.1f us/call  kernels(us): %s" % (N, what, 1e6 * wall,
               {k: round(1e3 * v[1] / v[0], 1) for k, v in prof.items()}), flush=True)
