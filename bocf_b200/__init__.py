@@ -5,7 +5,7 @@ CUDA kernels (bocf_b200/csrc) reached through a C ABI (include/bocf_b200.h).  No
 """
 from ._lib import load_library, launch_count, BocfError, NotPositiveDefiniteError, LIB_PATH  # noqa: F401
 from . import kern  # noqa: F401
-from .utility import Utility, ParameterDistribution  # noqa: F401
+from .utility import Utility, ParameterDistribution, CudaComposite  # noqa: F401
 from .model import multi_outputGP  # noqa: F401
 from .acquisitions import AcquisitionBase, uEI_noiseless, uPI, maEI, maPI, EI, PI  # noqa: F401
 from .optimization import (AcquisitionOptimizer, GeneralOptimizer, Design_space, Sequential,  # noqa: F401

@@ -5,6 +5,7 @@ RuntimeError is raised with the library's own message.
 """
 import ctypes
 import os
+import sys
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BOCF_LIB_PATH") or os.path.join(_HERE, "csrc", "libbocf_b200.so")   # override: kernel-variant experiments
@@ -12,6 +13,7 @@ _lib = None
 
 KERNELS = {"se": 0, "rbf": 1, "matern52": 2, "matern32": 3}
 COMPOSITES = {"sumsq_target": 0, "neg_sum_exp": 1, "exp_cos": 2, "rosen_composite": 3, "linear": 4}
+COMPOSITE_USER_BASE = 1024      # BOCF_U_USER: ids of composites registered with bocf_composite_register
 VARIANTS = {"ei_cf": 0, "pi_cf": 1, "ma_ei": 2, "ma_pi": 3, "mean_utility": 4, "psi": 5}
 
 EXPORTS = [
@@ -19,7 +21,7 @@ EXPORTS = [
     "bocf_model_create", "bocf_model_set_kernels", "bocf_model_destroy", "bocf_model_set_data", "bocf_model_set_hypers",
     "bocf_model_factorize", "bocf_model_get_factor", "bocf_model_n", "bocf_model_H",
     "bocf_model_set_scratch_limit", "bocf_posterior", "bocf_posterior_cov_point", "bocf_acq_eval", "bocf_acq_eval_host",
-    "bocf_utility_eval", "bocf_topk", "bocf_profile_enable", "bocf_profile_report",
+    "bocf_utility_eval", "bocf_utility_grad_eval", "bocf_composite_register", "bocf_topk", "bocf_profile_enable", "bocf_profile_report",
     "bocf_model_set_precision", "bocf_model_active_slices", "bocf_model_active_scheme", "bocf_model_chunk_candidates", "bocf_debug_split_gemm", "bocf_model_log_likelihood", "bocf_model_append_point",
 ]
 # name -> (enum bocf_precision, slices).  "splitN": both contractions on the N-plane scheme; "splitNM": variance on N,
@@ -79,6 +81,8 @@ def load_library():
                                   c_dp, c_dp, c_vp]
     lib.bocf_acq_eval_host.argtypes = lib.bocf_acq_eval.argtypes
     lib.bocf_utility_eval.argtypes = [i32, i32, c_dp, i64, c_dp, i32, i32, c_dp, c_vp]
+    lib.bocf_utility_grad_eval.argtypes = lib.bocf_utility_eval.argtypes
+    lib.bocf_composite_register.argtypes = [ctypes.c_char_p, i32, i32, ctypes.POINTER(i32)]
     lib.bocf_topk.argtypes = [c_dp, c_dp, i64, i32, i32, i64, c_dp, c_vp]
     lib.bocf_model_set_precision.argtypes = [c_vp, i32, i32, c_vp]
     lib.bocf_model_active_slices.argtypes = [c_vp]
@@ -96,6 +100,43 @@ def load_library():
             fn.restype = i32
     _lib = lib
     return lib
+
+
+_nvrtc = None
+
+
+def _nvrtc_candidates():
+    yield "libnvrtc.so.12"
+    for base in sys.path:                  # the copy bundled with the torch wheel, found without importing torch
+        yield os.path.join(base, "nvidia", "cuda_nvrtc", "lib", "libnvrtc.so.12")
+    for home in (os.environ.get("CUDA_HOME"), "/usr/local/cuda"):
+        if home:
+            yield os.path.join(home, "lib64", "libnvrtc.so.12")
+
+
+def preload_nvrtc():
+    """Load NVRTC with RTLD_GLOBAL, so the library's own dlopen("libnvrtc.so.12") at the first composite registration
+    finds it by soname even when it is not on the loader's search path."""
+    global _nvrtc
+    if _nvrtc is None:
+        for cand in _nvrtc_candidates():
+            if os.path.isabs(cand) and not os.path.exists(cand):
+                continue
+            try:
+                _nvrtc = ctypes.CDLL(cand, mode=ctypes.RTLD_GLOBAL)
+                break
+            except OSError:
+                continue
+    return _nvrtc
+
+
+def register_composite(source, m, theta_len):
+    """bocf_composite_register: compile a user composite for m outputs (theta_len -1 = m); returns its id."""
+    lib = load_library()
+    preload_nvrtc()
+    out = ctypes.c_int(-1)
+    check(lib.bocf_composite_register(source.encode("utf-8"), int(m), int(theta_len), ctypes.byref(out)))
+    return out.value
 
 
 def check(rc):

@@ -141,13 +141,14 @@ class AcquisitionBase(object):
                              % (L, w_h.size, f_h.shape))
         acq = np.empty((N, 1))
         dacq = np.empty((N, d)) if grad else None
+        cid = self.utility.composite_id(model.output_dim, model.device)
         with model._lock:
             # self-contained call (copies in, sweep, copies out, one synchronisation) on the handle's own stream: no
             # torch device / stream bookkeeping on this latency-bound path.  Everything it depends on (factor, digit
             # planes, base samples) was synchronised when it was produced.
             st = model._side_stream_ptr()
             _lib.check(model._lib.bocf_acq_eval_host(
-                model._handle, _lib.VARIANTS[variant], _lib.COMPOSITES[self.utility.composite],
+                model._handle, _lib.VARIANTS[variant], cid,
                 Xn.ctypes.data_as(ctypes.c_void_p), N, _ptr(Zt), S, th_p, L, theta.shape[1], w_p, f_p, f_h.shape[0], form,
                 acq.ctypes.data_as(ctypes.c_void_p), None if dacq is None else dacq.ctypes.data_as(ctypes.c_void_p), st))
         if self._sign < 0:
@@ -169,13 +170,14 @@ class AcquisitionBase(object):
             raise ValueError("need one weight and one incumbent column per utility parameter: L=%d, %d weights, f* %s"
                              % (L, w_h.size, f_h.shape))
         H_use = f_h.shape[0]
+        cid = self.utility.composite_id(model.output_dim, model.device)
         with model._lock, torch.cuda.device(model.device):
             acq = torch.empty((N,), dtype=torch.float64, device=model.device)
             dacq = torch.empty((N, d), dtype=torch.float64, device=model.device) if grad else None
             st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-            _lib.check(model._lib.bocf_acq_eval(model._handle, _lib.VARIANTS[variant],
-                                                _lib.COMPOSITES[self.utility.composite], _ptr(Xd), N, _ptr(Zt), S, th_p, L,
-                                                theta.shape[1], w_p, f_p, H_use, form, _ptr(acq), _ptr(dacq), st))
+            _lib.check(model._lib.bocf_acq_eval(model._handle, _lib.VARIANTS[variant], cid, _ptr(Xd), N, _ptr(Zt), S,
+                                                th_p, L, theta.shape[1], w_p, f_p, H_use, form, _ptr(acq), _ptr(dacq),
+                                                st))
             if self._sign < 0:
                 acq.neg_()
                 if dacq is not None:
@@ -294,11 +296,12 @@ class uEI_noiseless(AcquisitionBase):
         L, p = theta.shape
         th_h, th_p = _host(theta)
         n = fX.shape[1]
+        cid = self.utility.composite_id(model.output_dim, model.device)
         with torch.cuda.device(model.device):
             U = torch.empty((L, n), dtype=torch.float64, device=model.device)
             st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-            _lib.check(model._lib.bocf_utility_eval(_lib.COMPOSITES[self.utility.composite], model.output_dim,
-                                                    _ptr(fX.contiguous()), n, th_p, L, p, _ptr(U), st))
+            _lib.check(model._lib.bocf_utility_eval(cid, model.output_dim, _ptr(fX.contiguous()), n, th_p, L, p, _ptr(U),
+                                                    st))
             return U.max(dim=1).values.cpu().numpy()
 
     def _fstar(self, theta, per_hyper_sample=False):

@@ -113,6 +113,7 @@ class CBO(object):
                             "(CPU models are driven through oracle.cbo.CBO in the tests)")
         n_h = self._n_hyps()
         comp = self.utility.composite
+        self.utility.composite_id(model.output_dim, model.device)     # a CudaComposite: compiled and checked once
         if self.utility.linear:                                           # cbo.py:126-168
             if comp != "linear":
                 raise ValueError("Utility(linear=True) needs composite='linear'")

@@ -541,6 +541,20 @@ __global__ void utility_eval_kernel(int m, const double* __restrict__ Y, int64_t
   out[(int64_t)l * N + i] = U;
 }
 
+// out[l][j][i] = dU/dy_j (theta_l, Y[:, i]) = dphi_j (bocf_utility_grad_eval)
+template <int COMP>
+__global__ void utility_grad_eval_kernel(int m, const double* __restrict__ Y, int64_t N, const double* __restrict__ theta,
+                                         int L, int p, double* __restrict__ out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int l = blockIdx.y;
+  if (i >= N) return;
+  const double* th = theta + (int64_t)l * p;
+  for (int j = 0; j < m; ++j) {
+    const CompCtx c = comp_ctx<COMP>(th, j, m);
+    out[((int64_t)l * m + j) * N + i] = comp_dphi<COMP>(c, Y[(int64_t)j * N + i]);
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------
 // top-k (largest value, ties -> smaller index).  key order: a before b  <=>  va > vb || (va == vb && ia < ib)
 __device__ __forceinline__ bool key_before(double va, int64_t ia, double vb, int64_t ib) {
@@ -689,6 +703,7 @@ int launch_acq_chunk(const AcqParams& P, const ChunkBuffers& cb, int64_t Nvalid,
       set_error("mc acquisition: m exceeds MAXM");
       return -5;
     }
+    if (is_user_composite(P.composite)) return launch_mc_user(P, cb, Nvalid, acq, dacq, st);
     switch (P.composite) {
       case BOCF_U_SUMSQ_TARGET: return launch_mc_t<BOCF_U_SUMSQ_TARGET>(P, cb, Nvalid, acq, dacq, st);
       case BOCF_U_NEG_SUM_EXP: return launch_mc_t<BOCF_U_NEG_SUM_EXP>(P, cb, Nvalid, acq, dacq, st);
@@ -721,9 +736,28 @@ int launch_acq_chunk(const AcqParams& P, const ChunkBuffers& cb, int64_t Nvalid,
   return 0;
 }
 
+template <int COMP>
+static void launch_utility_grad_eval_t(dim3 grid, int m, const double* Y, int64_t N, const double* theta, int L, int p,
+                                       double* out, cudaStream_t st) {
+  utility_grad_eval_kernel<COMP><<<grid, 256, 0, st>>>(m, Y, N, theta, L, p, out);
+}
+
 int launch_utility_eval(int composite, int m, const double* Y, int64_t N, const double* theta, int L, int p,
-                        double* out, cudaStream_t st) {
+                        double* out, bool grad, cudaStream_t st) {
+  if (is_user_composite(composite)) return launch_utility_eval_user(composite, Y, N, theta, L, p, out, grad, st);
   dim3 grid((unsigned)ceil_div(N, 256), (unsigned)L);
+  if (grad) {
+    switch (composite) {
+      case BOCF_U_SUMSQ_TARGET: launch_utility_grad_eval_t<BOCF_U_SUMSQ_TARGET>(grid, m, Y, N, theta, L, p, out, st); break;
+      case BOCF_U_NEG_SUM_EXP: launch_utility_grad_eval_t<BOCF_U_NEG_SUM_EXP>(grid, m, Y, N, theta, L, p, out, st); break;
+      case BOCF_U_EXP_COS: launch_utility_grad_eval_t<BOCF_U_EXP_COS>(grid, m, Y, N, theta, L, p, out, st); break;
+      case BOCF_U_ROSEN_COMPOSITE: launch_utility_grad_eval_t<BOCF_U_ROSEN_COMPOSITE>(grid, m, Y, N, theta, L, p, out, st); break;
+      case BOCF_U_LINEAR: launch_utility_grad_eval_t<BOCF_U_LINEAR>(grid, m, Y, N, theta, L, p, out, st); break;
+      default: set_error("unknown composite"); return -1;
+    }
+    BOCF_LAUNCH_OK("utility_grad_eval_kernel");
+    return 0;
+  }
   switch (composite) {
     case BOCF_U_SUMSQ_TARGET: utility_eval_kernel<BOCF_U_SUMSQ_TARGET><<<grid, 256, 0, st>>>(m, Y, N, theta, L, p, out); break;
     case BOCF_U_NEG_SUM_EXP: utility_eval_kernel<BOCF_U_NEG_SUM_EXP><<<grid, 256, 0, st>>>(m, Y, N, theta, L, p, out); break;

@@ -701,8 +701,21 @@ int bocf_acq_eval(bocf_model* M, int variant, int composite, const double* Xc, i
     return BOCF_ERR_INVALID;
   }
   if (mc || marginal) {
-    const int need_p = (composite == BOCF_U_SUMSQ_TARGET || composite == BOCF_U_LINEAR) ? M->m
-                       : (composite == BOCF_U_ROSEN_COMPOSITE ? 1 : 0);
+    int need_p = (composite == BOCF_U_SUMSQ_TARGET || composite == BOCF_U_LINEAR) ? M->m
+                 : (composite == BOCF_U_ROSEN_COMPOSITE ? 1 : 0);
+    if (is_user_composite(composite)) {
+      int um = 0;
+      if (int rc = user_composite_info(composite, &um, &need_p)) return rc;
+      if (variant == BOCF_ACQ_PSI) {
+        set_error("bocf_acq_eval: a user-defined composite has no closed-form expectation: use BOCF_ACQ_MEAN_UTILITY");
+        return BOCF_ERR_UNSUPPORTED;
+      }
+      if (um != M->m) {
+        set_error("bocf_acq_eval: the composite was registered for " + std::to_string(um) + " outputs, the model has " +
+                  std::to_string(M->m));
+        return BOCF_ERR_INVALID;
+      }
+    }
     if (p < need_p) {
       set_error("bocf_acq_eval: theta has too few entries for this composite");
       return BOCF_ERR_INVALID;
@@ -820,11 +833,21 @@ int bocf_acq_eval_host(bocf_model* M, int variant, int composite, const double* 
   return rc;
 }
 
-int bocf_utility_eval(int composite, int m, const double* Y, int64_t N, const double* theta, int L, int p,
-                      double* out, void* stream) {
+static int utility_eval(const char* fn, int composite, int m, const double* Y, int64_t N, const double* theta, int L,
+                        int p, double* out, bool grad, void* stream) {
   if (!Y || !out || N < 0 || L < 1 || m < 1 || (p > 0 && !theta)) {
-    set_error("bocf_utility_eval: invalid arguments");
+    set_error(std::string(fn) + ": invalid arguments");
     return BOCF_ERR_INVALID;
+  }
+  if (is_user_composite(composite)) {
+    int um = 0, need_p = 0;
+    if (int rc = user_composite_info(composite, &um, &need_p)) return rc;
+    if (um != m || p < need_p) {
+      set_error(std::string(fn) + ": the composite was registered for " + std::to_string(um) + " outputs and " +
+                std::to_string(need_p) + " parameter entries (got m = " + std::to_string(m) + ", p = " +
+                std::to_string(p) + ")");
+      return BOCF_ERR_INVALID;
+    }
   }
   if (N == 0) return 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -836,13 +859,23 @@ int bocf_utility_eval(int composite, int m, const double* Y, int64_t N, const do
     set_error("H2D copy of theta failed");
     rc = BOCF_ERR_CUDA;
   }
-  if (!rc) rc = launch_utility_eval(composite, m, Y, N, dth, L, p, out, st);
+  if (!rc) rc = launch_utility_eval(composite, m, Y, N, dth, L, p, out, grad, st);
   if (cudaStreamSynchronize(st) != cudaSuccess && !rc) {
-    set_error("bocf_utility_eval: stream sync failed");
+    set_error(std::string(fn) + ": stream sync failed");
     rc = BOCF_ERR_CUDA;
   }
   dev_free(dth);
   return rc;
+}
+
+int bocf_utility_eval(int composite, int m, const double* Y, int64_t N, const double* theta, int L, int p,
+                      double* out, void* stream) {
+  return utility_eval("bocf_utility_eval", composite, m, Y, N, theta, L, p, out, false, stream);
+}
+
+int bocf_utility_grad_eval(int composite, int m, const double* Y, int64_t N, const double* theta, int L, int p,
+                           double* out, void* stream) {
+  return utility_eval("bocf_utility_grad_eval", composite, m, Y, N, theta, L, p, out, true, stream);
 }
 
 int bocf_topk(const double* acq, const double* Xc, int64_t N, int d, int k, int64_t index_offset, double* out_rec,

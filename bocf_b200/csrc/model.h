@@ -208,10 +208,21 @@ int launch_fused_grad_chunk(bocf_model* M, int h, const double* Xc, int64_t Nval
                             AcqParams P, double* acq, double* dacq, cudaStream_t st);
 int launch_acq_chunk(const AcqParams& P, const ChunkBuffers& cb, int64_t Nvalid, double* acq, double* dacq,
                      cudaStream_t st);
+// grad: out (L x m x N) = dU/dy_j instead of U
 int launch_utility_eval(int composite, int m, const double* Y, int64_t N, const double* theta, int L, int p,
-                        double* out, cudaStream_t st);
+                        double* out, bool grad, cudaStream_t st);
 int launch_topk(const double* acq, const double* Xc, int64_t N, int d, int k, int64_t index_offset,
                 double* out_rec, void* workspace, cudaStream_t st);
 uint64_t topk_workspace_bytes(int64_t N, int k);
+
+// ---- jit.cu -------------------------------------------------------------------------------------
+// user-defined composites (ids >= BOCF_U_USER, bocf_composite_register)
+bool is_user_composite(int composite);
+// registered outputs and parameter length (theta_len -1 resolved to m); BOCF_ERR_INVALID for an unknown id
+int user_composite_info(int composite, int* m, int* theta_len);
+int launch_mc_user(const AcqParams& P, const ChunkBuffers& cb, int64_t Nvalid, double* acq, double* dacq,
+                   cudaStream_t st);
+int launch_utility_eval_user(int composite, const double* Y, int64_t N, const double* theta, int L, int p, double* out,
+                             bool grad, cudaStream_t st);
 
 }  // namespace bocf

@@ -18,6 +18,7 @@ import torch
 
 from . import _lib
 from . import kern as _kern
+from .utility import composite_id
 
 
 def _ptr(t):
@@ -341,7 +342,8 @@ class multi_outputGP(object):
 
     def expected_utility(self, X, composite, parameter, n_hyps, Z=None, grad=False):
         """sum over the first n_hyps hyper-samples of the expected composite utility at X under the NOISELESS posterior,
-        NOT normalised -- the objective cbo._current_marginal_argmax maximises (cbo.py:121-235):
+        NOT normalised -- the objective cbo._current_marginal_argmax maximises (cbo.py:121-235).  `composite` is a
+        catalogued name or a CudaComposite (MC branch only: it has no closed form):
           Z is None : closed form psi(theta, mu, var) (cbo.py:170-198; LINEAR = the posterior-mean branch :126-168)
           Z (S, m)  : sum_s U(theta, mu + sqrt(var) Z_s) with the pathwise gradient (cbo.py:203-231).
         Returns (value (N,), gradient (N, d) or None) as numpy (CUDA tensors for tensor input)."""
@@ -351,6 +353,7 @@ class multi_outputGP(object):
         ones = np.ones(1)
         zeros = np.zeros((int(n_hyps), 1))
         variant = "psi" if Z is None else "mean_utility"
+        cid = composite_id(composite, self.output_dim)
         with self._lock, torch.cuda.device(self.device):
             Zt, S = None, 0
             if Z is not None:
@@ -360,7 +363,7 @@ class multi_outputGP(object):
             val = torch.empty((N,), dtype=torch.float64, device=self.device)
             g = torch.empty((N, d), dtype=torch.float64, device=self.device) if grad else None
             st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-            _lib.check(self._lib.bocf_acq_eval(self._handle, _lib.VARIANTS[variant], _lib.COMPOSITES[composite], _ptr(Xd), N,
+            _lib.check(self._lib.bocf_acq_eval(self._handle, _lib.VARIANTS[variant], cid, _ptr(Xd), N,
                                                _ptr(Zt), S, theta.ctypes.data_as(ctypes.c_void_p), 1, theta.shape[1],
                                                ones.ctypes.data_as(ctypes.c_void_p), zeros.ctypes.data_as(ctypes.c_void_p),
                                                int(n_hyps), 0, _ptr(val), _ptr(g), st))

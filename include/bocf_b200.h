@@ -50,8 +50,28 @@ enum bocf_composite {
   BOCF_U_NEG_SUM_EXP = 1,      /* -sum_j exp(y_j)                 test_2a.py:60-65   p = 0 */
   BOCF_U_EXP_COS = 2,          /* -sum_j c_j e^{-y_j/pi}cos(pi y_j) test_3a.py:53-67 p = 0 */
   BOCF_U_ROSEN_COMPOSITE = 3,  /* -sum_{j<m/2} (theta-y_j)^2+100 y_{j+m/2}^2  test_5a.py:48-59 p = 1 */
-  BOCF_U_LINEAR = 4            /* theta . y                       test_1b.py:89-93   p = m */
+  BOCF_U_LINEAR = 4,           /* theta . y                       test_1b.py:89-93   p = m */
+  BOCF_U_USER = 1024           /* first id bocf_composite_register hands out                   */
 };
+
+/* User-defined composites.  bocf_composite_register compiles CUDA C++ source (fp64) that defines
+ *
+ *   __device__ double bocf_U (const double* theta, const double* y);               // y[0 .. BOCF_M)
+ *   __device__ void   bocf_dU(const double* theta, const double* y, double* grad); // grad[j] = dU/dy_j, j < BOCF_M
+ *
+ * for m outputs: the library defines BOCF_M = m before the source.  theta points at ONE utility parameter of
+ * theta_len entries (-1: one entry per output, theta_len = m).  The source is compiled with NVRTC for sm_100a, without
+ * host or toolkit headers: the CUDA math functions NVRTC provides built in (exp, log, sin, sqrt, fma, ...) are
+ * available; constants such as pi are written out.  Every entry that takes a composite accepts the returned id: the
+ * MC variants of bocf_acq_eval / bocf_acq_eval_host (EI_CF, PI_CF, MEAN_UTILITY; not PSI, which needs a closed form),
+ * bocf_utility_eval and bocf_utility_grad_eval, each with the registered m and p >= theta_len.
+ *
+ * The call compiles immediately (no GPU needed) and returns in *composite_out an id >= BOCF_U_USER; registering the
+ * same (source, m, theta_len) again returns the same id.  The registry is process-wide and thread-safe; the compiled
+ * module is loaded on each device at its first launch there.  Returns BOCF_ERR_INVALID for a source that does not
+ * compile (the NVRTC log is in bocf_last_error()) or m outside [1, 64], and BOCF_ERR_UNSUPPORTED when libnvrtc.so.12
+ * cannot be loaded (it is dlopen'ed at the first registration). */
+int bocf_composite_register(const char* source, int m, int theta_len, int* composite_out);
 
 /* Acquisition variants. */
 enum bocf_acq_variant {
@@ -209,6 +229,9 @@ int bocf_acq_eval_host(bocf_model* mdl, int variant, int composite, const double
 /* U(theta_l, Y[:, i]) for a batch: Y [dev] m x N -> out [dev] L x N.  Used for f* (uEI_noiseless.py:76). */
 int bocf_utility_eval(int composite, int m, const double* Y, int64_t N, const double* theta, int L,
                       int p, double* out, void* stream);
+/* Its gradient twin: out [dev] L x m x N, out[l][j][i] = dU/dy_j (theta_l, Y[:, i]). */
+int bocf_utility_grad_eval(int composite, int m, const double* Y, int64_t N, const double* theta, int L,
+                           int p, double* out, void* stream);
 
 /* Local top-k of the LARGEST acq values (anchor selection, anchor_points_generator.py:59-64 with
  * f = -acq).  Ties break on the smaller candidate index.  out_val [dev] k, out_idx [dev] k (int64,
