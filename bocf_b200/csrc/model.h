@@ -156,6 +156,9 @@ struct ChunkBuffers {          // scratch views for one candidate chunk (Nc rows
   double* kpart = nullptr;     // K-split partial sums of mean / dmean for small chunks (posterior.cu: kstar_ksplit)
   double* wa = nullptr;        // split mode, fused gradient path: m x Nc weights of the mean gradient      (acq.cu)
   double* wb = nullptr;        //                                  m x Nc weights of the variance gradient
+  int* unit_flags = nullptr;   //   m x RTv  unit (output j, candidate tile rt) has a non-zero weight (index j * RTv + rt)
+  int* unit_list = nullptr;    //   ids j * RTv + rt of the flagged units, ascending
+  int* unit_count = nullptr;   //   length of unit_list
 };
 int kstar_ksplit(const bocf_model* M, int64_t Nc);
 uint64_t kstar_part_bytes(const bocf_model* M, int64_t Nc);

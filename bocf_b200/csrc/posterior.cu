@@ -561,18 +561,73 @@ static int launch_kstar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, 
   return 0;
 }
 
+// ===================================================================================================
+// Active units of the fused gradient's second contraction.  A unit (output j, candidate tile rt) whose gradient weights
+// WA, WB are all exactly zero contributes exactly zero to the acquisition gradient (EI-CF: no base sample of its
+// candidates passes the strict indicator U > f*).  Uniformly spread candidates almost never improve on the incumbent, so
+// most units of a sweep are in this case and the EPI_DACQ contraction walks only the flagged ones.  The weights' producer
+// does not matter (mc_acq_kernel, mc_acq_user_kernel, ma_acq_kernel).  A NaN weight counts as non-zero.
+// flags[j * RTv + rt], one warp per unit; only valid candidates (i < Nvalid) are read.
+__global__ void active_units_flag_kernel(const double* __restrict__ wa, const double* __restrict__ wb, int64_t Nc,
+                                         int64_t Nvalid, int rtv, int units, int* __restrict__ flags) {
+  const int unit = (int)blockIdx.x * (blockDim.x >> 5) + (int)(threadIdx.x >> 5);
+  if (unit >= units) return;
+  const int lane = threadIdx.x & 31;
+  const int j = unit / rtv, rt = unit - j * rtv;
+  bool act = false;
+#pragma unroll
+  for (int r = lane; r < CT; r += 32) {
+    const int64_t i = (int64_t)rt * CT + r;
+    if (i < Nvalid) act |= !(wa[(int64_t)j * Nc + i] == 0.0) || !(wb[(int64_t)j * Nc + i] == 0.0);
+  }
+  act = __any_sync(0xffffffffu, act);
+  if (lane == 0) flags[unit] = act ? 1 : 0;
+}
+
+// The ids of the flagged units in ascending order and their number: one block of 1024 threads, 1024 flags per trip.
+__global__ void __launch_bounds__(1024) active_units_list_kernel(const int* __restrict__ flags, int units,
+                                                                 int* __restrict__ list, int* __restrict__ count) {
+  __shared__ int s_warp[32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int base = 0;
+  for (int u0 = 0; u0 < units; u0 += 1024) {
+    const int u = u0 + (int)threadIdx.x;
+    const bool f = (u < units) && flags[u] != 0;
+    const unsigned b = __ballot_sync(0xffffffffu, f);
+    if (lane == 0) s_warp[warp] = __popc(b);
+    __syncthreads();
+    const int wc = s_warp[lane];                           // every warp scans the 32 warp counts itself
+    int incl = wc;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int t = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += t;
+    }
+    const int before = __shfl_sync(0xffffffffu, incl - wc, warp);
+    if (f) list[base + before + __popc(b & ((1u << lane) - 1u))] = u;
+    base += __shfl_sync(0xffffffffu, incl, 31);
+    __syncthreads();                                       // s_warp is rewritten by the next trip
+  }
+  if (threadIdx.x == 0) *count = base;
+}
+
 // sum over outputs and partials of the fused gradient:  dacq[i][q] (+)= sum_j (xs_jq S0_j - ACC_jq) / l_jq
-// (S0 / ACC: the weighted sums the EPI_DACQ epilogue leaves per output, split_gemm.cu)
+// (S0 / ACC: the weighted sums the EPI_DACQ epilogue leaves per output, split_gemm.cu).  Units without a flag were not
+// computed: they contribute exactly zero, and their partial slots hold whatever an earlier chunk left there.
 __global__ void finalize_grad_kernel(const double* __restrict__ part_dvar, const double* __restrict__ part_s0,
-                                     const OutHyp* __restrict__ hyp, int64_t Nc, int64_t Nvalid, int nparts, int m, int d,
-                                     int h, const double* __restrict__ Xc, int accumulate, double* __restrict__ dacq) {
+                                     const int* __restrict__ unit_flags, const OutHyp* __restrict__ hyp, int64_t Nc,
+                                     int64_t Nvalid, int nparts, int m, int d, int h, const double* __restrict__ Xc,
+                                     int accumulate, double* __restrict__ dacq) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= Nvalid * d) return;
   const int64_t i = idx / d;
   const int q = (int)(idx - i * d);
+  const int rtv = (int)((Nvalid + CT - 1) / CT);
+  const int* flag = unit_flags + i / CT;
   const double x = Xc[i * d + q];
   double g = 0.0;
   for (int j = 0; j < m; ++j) {
+    if (flag[j * rtv] == 0) continue;
     const OutHyp& hp = hyp[h * m + j];
     double acc = 0.0, s0 = 0.0;
     for (int t = 0; t < nparts; ++t) {
@@ -587,8 +642,10 @@ __global__ void finalize_grad_kernel(const double* __restrict__ part_dvar, const
 // The same sum for tiny batches (the L-BFGS rounds: <= 128 candidates), where one thread per (candidate, dimension)
 // walking m x nparts partials serially is pure latency (~50 us at m = 16, 12 partials): a WARP per (candidate, dimension),
 // lanes striding over the (output, partial) pairs -- the sum is linear in them -- then one shuffle reduction.
+// (one candidate tile: the unit flags are unit_flags[j])
 __global__ void __launch_bounds__(256) finalize_grad_small_kernel(const double* __restrict__ part_dvar,
                                                                   const double* __restrict__ part_s0,
+                                                                  const int* __restrict__ unit_flags,
                                                                   const OutHyp* __restrict__ hyp, int64_t Nc, int64_t Nvalid,
                                                                   int nparts, int m, int d, int h,
                                                                   const double* __restrict__ Xc, int accumulate,
@@ -602,6 +659,7 @@ __global__ void __launch_bounds__(256) finalize_grad_small_kernel(const double* 
   double g = 0.0;
   for (int p = lane; p < m * nparts; p += 32) {
     const int j = p / nparts;                                  // p = j * nparts + t
+    if (unit_flags[j] == 0) continue;
     const double il = 1.0 / hyp[h * m + j].ls[q];
     g += (x * il * part_s0[(int64_t)p * Nc + i] - part_dvar[((int64_t)p * Nc + i) * d + q]) * il;
   }
@@ -611,9 +669,9 @@ __global__ void __launch_bounds__(256) finalize_grad_small_kernel(const double* 
 
 // Fused acquisition-gradient sweep of one chunk and one hyper-sample (EI-CF / mean-utility with gradients, tensor-core
 // contraction mode): K* (mean, digit planes, G*; no mean gradient) -> first contraction -> variance -> MC forward pass
-// leaving the value and the per-(candidate, output) gradient weights WA, WB -> second contraction whose epilogue
-// contracts G* (WA alpha - 2 WB Wt) against the training inputs -> sum over outputs.  The per-output mean / variance
-// gradients (2 m d doubles per candidate) are never formed.
+// leaving the value and the per-(candidate, output) gradient weights WA, WB -> the units with a non-zero weight ->
+// second contraction over those units, whose epilogue contracts G* (WA alpha - 2 WB Wt) against the training inputs ->
+// sum over outputs.  The per-output mean / variance gradients (2 m d doubles per candidate) are never formed.
 int launch_fused_grad_chunk(bocf_model* M, int h, const double* Xc, int64_t Nvalid, int noiseless, const ChunkBuffers& cb,
                             AcqParams P, double* acq, double* dacq, cudaStream_t st) {
   if (int rc = launch_kstar(M, h, Xc, Nvalid, 2, cb, st)) return rc;
@@ -629,15 +687,27 @@ int launch_fused_grad_chunk(bocf_model* M, int h, const double* Xc, int64_t Nval
   P.wa = cb.wa;
   P.wb = cb.wb;
   if (int rc = launch_acq_chunk(P, cb, Nvalid, acq, nullptr, st)) return rc;
+  {
+    const int rtv = (int)ceil_div(Nvalid, CT);
+    const int units = M->m * rtv;
+    ProfScope ps("active_units_kernel", st);
+    active_units_flag_kernel<<<(unsigned)ceil_div(units, 8), 256, 0, st>>>(cb.wa, cb.wb, cb.Nc, Nvalid, rtv, units,
+                                                                           cb.unit_flags);
+    BOCF_LAUNCH_OK("active_units_flag_kernel");
+    active_units_list_kernel<<<1, 1024, 0, st>>>(cb.unit_flags, units, cb.unit_list, cb.unit_count);
+    BOCF_LAUNCH_OK("active_units_list_kernel");
+  }
   if (int rc = launch_split_dvar(M, h, Xc, Nvalid, cb, true, st)) return rc;
   {
     ProfScope ps("finalize_kernel", st);
     if (Nvalid <= 128)
-      finalize_grad_small_kernel<<<(unsigned)ceil_div(Nvalid * M->d, 8), 256, 0, st>>>(cb.part_dvar, cb.part_s0, M->hyp, cb.Nc,
-                                                                                     Nvalid, split_partials_dvar(M, cb.Nc),
-                                                                                     M->m, M->d, h, Xc, P.accumulate, dacq);
+      finalize_grad_small_kernel<<<(unsigned)ceil_div(Nvalid * M->d, 8), 256, 0, st>>>(cb.part_dvar, cb.part_s0, cb.unit_flags,
+                                                                                     M->hyp, cb.Nc, Nvalid,
+                                                                                     split_partials_dvar(M, cb.Nc), M->m, M->d,
+                                                                                     h, Xc, P.accumulate, dacq);
     else
-      finalize_grad_kernel<<<(unsigned)ceil_div(Nvalid * M->d, 256), 256, 0, st>>>(cb.part_dvar, cb.part_s0, M->hyp, cb.Nc, Nvalid,
+      finalize_grad_kernel<<<(unsigned)ceil_div(Nvalid * M->d, 256), 256, 0, st>>>(cb.part_dvar, cb.part_s0, cb.unit_flags,
+                                                                                 M->hyp, cb.Nc, Nvalid,
                                                                                  split_partials_dvar(M, cb.Nc), M->m, M->d, h,
                                                                                  Xc, P.accumulate, dacq);
     BOCF_LAUNCH_OK("finalize_grad_kernel");

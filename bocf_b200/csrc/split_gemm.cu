@@ -153,6 +153,10 @@ struct GemmParams {
   const OutHyp* hyp;
   int d, n16, n_pad;
   int np;                  // parts per candidate tile
+  // DACQ: the units (j, rt) to walk, as ids j * RTv + rt in ascending order, and their number (active_units_kernel,
+  // posterior.cu).  nullptr: every unit.
+  const int* unit_list;
+  const int* unit_count;
 };
 
 // Work decomposition.  A UNIT is (output j, candidate tile rt, part p of NP): the column tiles ct = p, p+NP, ... of one
@@ -186,11 +190,14 @@ struct TileInfo {
 // Walks the column tiles this CTA owns: units cta, cta + grid, ... and inside a unit the tiles ct = p, p + NP, ...
 // The (output, candidate tile, part) decode costs integer divisions, so it is done once per unit; advancing inside a
 // unit is additions only (every role of the kernel walks the same sequence, the epilogue one tile ahead as well).
-template <int NT>
+// LIST (EPI_DACQ): the (output, candidate tile) pairs come from P.unit_list, each still split into the same NP parts,
+// so a listed unit is computed exactly as in the dense walk; the grid stays what the host sized for the dense walk and
+// CTAs left without a unit fall through.
+template <int NT, bool LIST>
 struct TileWalk {
   int u, units, j, rt, p, ct;
   __device__ __forceinline__ void start(const GemmParams& P) {
-    units = P.m * P.RTv * P.np;
+    units = (LIST && P.unit_list != nullptr) ? __ldg(P.unit_count) * P.np : P.m * P.RTv * P.np;
     u = (int)blockIdx.x - (int)gridDim.x;
     ct = P.nct;                                            // forces the first next() to open a unit
     j = rt = p = 0;
@@ -201,10 +208,18 @@ struct TileWalk {
     while (ct >= P.nct) {                                  // open the next unit that has at least one column tile
       u += (int)gridDim.x;
       if (u >= units) return false;
-      j = u / (P.RTv * P.np);
-      const int r = u - j * (P.RTv * P.np);
-      rt = r / P.np;
-      p = r - rt * P.np;
+      if (LIST && P.unit_list != nullptr) {
+        const int e = u / P.np;
+        p = u - e * P.np;
+        const int id = __ldg(P.unit_list + e);
+        j = id / P.RTv;
+        rt = id - j * P.RTv;
+      } else {
+        j = u / (P.RTv * P.np);
+        const int r = u - j * (P.RTv * P.np);
+        rt = r / P.np;
+        p = r - rt * P.np;
+      }
       ct = p;
       first = true;
     }
@@ -377,7 +392,7 @@ __global__ void __launch_bounds__(Cfg<SCH, DP>::NTHREADS, 1) split_gemm_kernel(c
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      TileWalk<NT> walk;
+      TileWalk<NT, EPI == EPI_DACQ> walk;
       walk.start(P);
       TileInfo ti;
       while (walk.next(P, ti)) {
@@ -408,7 +423,7 @@ __global__ void __launch_bounds__(Cfg<SCH, DP>::NTHREADS, 1) split_gemm_kernel(c
     int stage = 0;
     uint32_t phase = 0;
     int it = 0;
-    TileWalk<NT> walk;
+    TileWalk<NT, EPI == EPI_DACQ> walk;
     walk.start(P);
     TileInfo ti;
     while (walk.next(P, ti)) {
@@ -479,7 +494,7 @@ __global__ void __launch_bounds__(Cfg<SCH, DP>::NTHREADS, 1) split_gemm_kernel(c
         }
       }
     };
-    TileWalk<NT> walk;
+    TileWalk<NT, EPI == EPI_DACQ> walk;
     walk.start(P);
     TileInfo ti, tnext;
     bool have = walk.next(P, tnext);
@@ -954,6 +969,7 @@ uint64_t split_chunk_bytes_per_candidate(const bocf_model* M, bool grad, int64_t
     per += (uint64_t)M->m * split_partials_dvar(M, Nc) * (M->d + 1) * 8;  // part_dvar, part_s0
     per += 2ull * M->m * M->d * 8;                      // dmean, dvar
     per += 2ull * M->m * 8;                             // wa, wb (fused gradient path)
+    per += (2ull * M->m * 4 + sg::TM - 1) / sg::TM;     // unit flags and unit list: one int each per (output, tile)
   }
   return per;
 }
@@ -981,6 +997,9 @@ void split_carve_chunk(const bocf_model* M, void* base, int64_t Nc, bool grad, C
     cb->dvar = reinterpret_cast<double*>(take((uint64_t)M->m * Nc * M->d * 8));
     cb->wa = reinterpret_cast<double*>(take((uint64_t)M->m * Nc * 8));
     cb->wb = reinterpret_cast<double*>(take((uint64_t)M->m * Nc * 8));
+    cb->unit_flags = reinterpret_cast<int*>(take((uint64_t)M->m * (Nc / sg::TM) * 4));
+    cb->unit_list = reinterpret_cast<int*>(take((uint64_t)M->m * (Nc / sg::TM) * 4 + 4));
+    cb->unit_count = cb->unit_list + M->m * (Nc / sg::TM);
   } else {
     cb->GsT = cb->part_dvar = cb->dmean = cb->dvar = nullptr;
     cb->A2 = nullptr;
@@ -1040,6 +1059,8 @@ int launch_split_dvar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, co
     P.alpha = M->alpha;
     P.wa = cb.wa;
     P.wb = cb.wb;
+    P.unit_list = cb.unit_list;
+    P.unit_count = cb.unit_count;
   }
   if (M->nct2 < P.np) {
     BOCF_CUDA_OK(cudaMemsetAsync(cb.part_dvar, 0, sizeof(double) * M->m * split_partials_dvar(M, cb.Nc) * cb.Nc * M->d, st));
