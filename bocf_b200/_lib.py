@@ -22,7 +22,7 @@ EXPORTS = [
     "bocf_model_factorize", "bocf_model_get_factor", "bocf_model_n", "bocf_model_H",
     "bocf_model_set_scratch_limit", "bocf_posterior", "bocf_posterior_cov_point", "bocf_acq_eval", "bocf_acq_eval_host",
     "bocf_utility_eval", "bocf_utility_grad_eval", "bocf_composite_register", "bocf_topk", "bocf_profile_enable", "bocf_profile_report",
-    "bocf_model_set_precision", "bocf_model_active_slices", "bocf_model_active_scheme", "bocf_model_chunk_candidates", "bocf_debug_split_gemm", "bocf_model_log_likelihood", "bocf_model_append_point",
+    "bocf_model_set_precision", "bocf_model_active_slices", "bocf_model_active_scheme", "bocf_model_chunk_candidates", "bocf_model_sweep_stats", "bocf_debug_split_gemm", "bocf_model_log_likelihood", "bocf_model_append_point",
 ]
 # name -> (enum bocf_precision, slices).  "splitN": both contractions on the N-plane scheme; "splitNM": variance on N,
 # variance gradient on M <= N planes (include/bocf_b200.h).
@@ -89,6 +89,7 @@ def load_library():
     lib.bocf_model_active_scheme.argtypes = [c_vp]
     lib.bocf_model_chunk_candidates.argtypes = [c_vp, i64, i32]
     lib.bocf_model_chunk_candidates.restype = i64
+    lib.bocf_model_sweep_stats.argtypes = [c_vp, ctypes.POINTER(i64), ctypes.POINTER(i64)]
     lib.bocf_debug_split_gemm.argtypes = [c_dp, c_dp, i32, i32, i32, i32, i32, c_dp, c_vp]
     lib.bocf_model_log_likelihood.argtypes = [c_vp, c_dp, c_dp, c_dp, c_dp, c_vp]
     lib.bocf_model_append_point.argtypes = [c_vp, c_dp, c_dp, c_vp]

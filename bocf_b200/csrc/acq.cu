@@ -85,6 +85,138 @@ __device__ __forceinline__ double comp_dphi(const CompCtx& c, double y) {
   }
 }
 
+// Upper bound of phi_j over the segment [lo, hi] (lo <= hi), and for LINEAR the magnitude max |phi_j| over it (the other
+// three are <= 0 everywhere: their magnitude is -bound, formed by the caller).  Exact maxima of the segment, evaluated with
+// the rounding error prune_bound_kernel's margin accounts for.
+template <int COMP>
+__device__ __forceinline__ double comp_seg_max(const CompCtx& c, double lo, double hi, double& mag) {
+  mag = 0.0;
+  if (COMP == BOCF_U_SUMSQ_TARGET || (COMP == BOCF_U_ROSEN_COMPOSITE && c.lower == 1)) {
+    // -(distance from the target to the segment)^2; the negated compares let a NaN through
+    const double d1 = lo - c.th, d2 = c.th - hi;
+    const double dist = !(d1 <= 0.0) ? d1 : (!(d2 <= 0.0) ? d2 : 0.0);
+    return -(dist * dist);
+  } else if (COMP == BOCF_U_ROSEN_COMPOSITE) {
+    if (c.lower != 0) return 0.0;
+    const double dist = !(lo <= 0.0) ? lo : (!(hi >= 0.0) ? -hi : 0.0);
+    return -(100.0 * (dist * dist));
+  } else if (COMP == BOCF_U_NEG_SUM_EXP) {
+    return -exp(lo);
+  } else {                                                    // LINEAR
+    mag = fabs(c.th) * fmax(fabs(lo), fabs(hi));
+    return c.th * ((c.th >= 0.0) ? hi : lo);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Survivor flags of the pruned EI-CF / PI-CF sweep (bocf_acq_eval).  mc_acq_kernel forms, per base sample s,
+// U_s = sum_j phi_j(mu_j + sigma_j z_sj) with sigma_j^2 the posterior variance (noise added, clipped at 1e-10), and a
+// candidate contributes nothing -- value, gradient weights, PI count -- unless some U_s > f* (PI: f* + 1e-6).  Since the
+// posterior variance never exceeds the prior one, sigma_j <= smax_j = sqrt(max(sigma_f,j^2 + noise_j, 1e-10)), so
+//   U_s <= UB_s = sum_j max_{t in [0, 1]} phi_j(mu_j + t smax_j z_sj),
+// a maximum over the segment between mu_j and mu_j + smax_j z_sj with a closed form (comp_seg_max).  A candidate is
+// pruned when UB_s + margin <= f* for every hyper-sample, utility parameter and base sample; flags[i] = 1 keeps it.  mu is
+// the mean-only pass's, bitwise the mean the sweep uses (posterior.cu); Zt, theta and f* are the sweep's own device slots.
+//
+// Why the floating-point comparison is safe (u = 2^-53, gamma_k = k u / (1 - k u)):
+//  * The segment holds the sweep's y.  mc_acq_kernel computes y = fl(mu + sigma z), contracted to one FMA or not, with
+//    sigma = sqrt(var) correctly rounded; its var <= max((sigma_f^2 + noise)(1 + u), 1e-10), so sigma <= smax (1 + 3.1 u).
+//    Here smax is inflated by 2^-47 (>= 14 u after rounding), so with P = smax z the sweep's exact sigma z lies strictly
+//    between 0 and fl(P), and by monotonicity of rounding y lies between mu and e = fl(mu + fl(P)).  e is formed with
+//    __dmul_rn / __dadd_rn so the compiler cannot contract it.  Hence phi_j(y_j) <= the exact maximum over [lo, hi].
+//  * SUMSQ_TARGET, ROSEN, NEG_SUM_EXP: every phi_j <= 0.  Each term of the sweep has a relative error <= gamma_3 (a
+//    subtraction and a square, or exp within 1 ulp, fused or not) and the sum over m terms adds gamma_(m-1) of the sum of
+//    magnitudes, so U_s(computed) <= (1 - gamma_(m+2)) U_s(exact) <= (1 - gamma_(m+2)) UB_s(exact).  The bound here is
+//    evaluated the same way, UB(computed) = UB(exact)(1 + eta), |eta| <= gamma_(m+2), both <= 0, which gives
+//    U_s(computed) <= UB + 2 gamma_(m+2) |UB| (computed UB).
+//  * LINEAR: the sweep and the bound each err by <= gamma_m sum_j |theta_j| max(|lo_j|, |hi_j|) = gamma_m MAG, so
+//    U_s(computed) <= UB + 2 gamma_m MAG / (1 - gamma_m) with MAG as computed here.
+//  The margin is (4 m + 16) u MAG (MAG = -UB for the first three), over twice what is needed, which also covers the
+//  rounding of UB + margin itself; the 1e-300 added to it covers results in the subnormal range, where errors are
+//  absolute (<= m * 2^-1072 in all).  A NaN anywhere (input, mean, theta, f*) fails the <= and keeps the candidate.
+constexpr int PB_WARPS = 8;
+constexpr int PB_MCB = 4;      // candidates per warp (each base sample loaded is applied to all of them)
+constexpr int PB_MCU = 4;      // sample groups per trip
+// (LINEAR carries the magnitude sums as well, NEG_SUM_EXP sixteen inlined exp: one block per SM keeps them in registers)
+template <int COMP>
+__global__ void __launch_bounds__(PB_WARPS * 32, (COMP == BOCF_U_LINEAR || COMP == BOCF_U_NEG_SUM_EXP) ? 1 : 2)
+    prune_bound_kernel(
+    const double* __restrict__ mean, int64_t Nc, int64_t Nvalid, int m, const OutHyp* __restrict__ hyp,
+    const double* __restrict__ Zt, int S, const double* __restrict__ theta, int L, int p,
+    const double* __restrict__ fstar, int pi, int first, uint8_t* __restrict__ flags) {
+  __shared__ double s_mu[PB_WARPS][MAXM][PB_MCB];
+  __shared__ double s_sd[MAXM];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int j = threadIdx.x; j < m; j += blockDim.x)
+    s_sd[j] = sqrt(fmax(hyp[j].variance + hyp[j].noise, 1e-10)) * (1.0 + 0x1p-47);
+  const int64_t i0 = ((int64_t)blockIdx.x * PB_WARPS + warp) * PB_MCB;
+  const int nc = (i0 < Nvalid) ? (int)min((int64_t)PB_MCB, Nvalid - i0) : 0;
+  for (int idx = lane; idx < m * PB_MCB && nc > 0; idx += 32) {
+    const int j = idx / PB_MCB, c = idx - j * PB_MCB;
+    s_mu[warp][j][c] = mean[(int64_t)j * Nc + i0 + min(c, nc - 1)];    // ragged tail: replicate the last candidate
+  }
+  __syncthreads();
+  if (nc == 0) return;
+  const double cm = (4.0 * m + 16.0) * 0x1p-53;
+  bool live[PB_MCB];                                        // warp-uniform
+#pragma unroll
+  for (int c = 0; c < PB_MCB; ++c) live[c] = (c >= nc);     // replicas count as decided
+  bool done = false;
+  for (int l = 0; l < L && !done; ++l) {
+    const double* th = theta + (int64_t)l * p;
+    const double fs = pi ? fstar[l] + 1e-6 : fstar[l];     // as mc_acq_kernel
+#pragma unroll 1
+    for (int s0 = 0; s0 < S && !done; s0 += 32 * PB_MCU) {
+      double ub[PB_MCB][PB_MCU], mg[PB_MCB][PB_MCU];
+#pragma unroll
+      for (int c = 0; c < PB_MCB; ++c)
+#pragma unroll
+        for (int u = 0; u < PB_MCU; ++u) ub[c][u] = mg[c][u] = 0.0;
+      for (int j = 0; j < m; ++j) {
+        const CompCtx cx = comp_ctx<COMP>(th, j, m);
+        const double sd = s_sd[j];
+        const double* zr = Zt + (int64_t)j * S + s0 + lane;
+        double z[PB_MCU];
+#pragma unroll
+        for (int u = 0; u < PB_MCU; ++u) z[u] = (s0 + u * 32 + lane < S) ? zr[u * 32] : 0.0;
+#pragma unroll
+        for (int c = 0; c < PB_MCB; ++c) {
+          const double mu = s_mu[warp][j][c];
+#pragma unroll
+          for (int u = 0; u < PB_MCU; ++u) {
+            const double e = __dadd_rn(mu, __dmul_rn(sd, z[u]));
+            const bool up = z[u] >= 0.0;
+            double mag;
+            ub[c][u] += comp_seg_max<COMP>(cx, up ? mu : e, up ? e : mu, mag);
+            if (COMP == BOCF_U_LINEAR) mg[c][u] += mag;
+          }
+        }
+      }
+#pragma unroll
+      for (int c = 0; c < PB_MCB; ++c) {
+        bool any = false;
+#pragma unroll
+        for (int u = 0; u < PB_MCU; ++u) {
+          const double mag = (COMP == BOCF_U_LINEAR) ? mg[c][u] : -ub[c][u];
+          if (s0 + u * 32 + lane < S) any |= !(ub[c][u] + fma(cm, mag, 1e-300) <= fs);
+        }
+        live[c] = live[c] || __any_sync(0xffffffffu, any);
+      }
+      done = true;
+#pragma unroll
+      for (int c = 0; c < PB_MCB; ++c) done = done && live[c];
+    }
+  }
+  if (lane < nc) {
+    bool v = false;
+#pragma unroll
+    for (int c = 0; c < PB_MCB; ++c)
+      if (c == lane) v = live[c];
+    const int64_t i = i0 + lane;
+    flags[i] = (uint8_t)((first ? 0 : flags[i]) | (v ? 1 : 0));
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------
 constexpr int MC_WARPS = 8;
 constexpr int MCU = 4;         // sample groups per trip (independent base-sample loads in flight per lane)
@@ -733,6 +865,199 @@ int launch_acq_chunk(const AcqParams& P, const ChunkBuffers& cb, int64_t Nvalid,
   }
 #undef BOCF_MA_ARGS
   BOCF_LAUNCH_OK("ma_acq_kernel");
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// pruned sweep (bocf_acq_eval): bound, survivor list, gather, scatter
+bool prune_supported(int variant, int composite) {
+  return (variant == BOCF_ACQ_EI_CF || variant == BOCF_ACQ_PI_CF) &&
+         (composite == BOCF_U_SUMSQ_TARGET || composite == BOCF_U_ROSEN_COMPOSITE || composite == BOCF_U_NEG_SUM_EXP ||
+          composite == BOCF_U_LINEAR);
+}
+
+int launch_prune_bound(const AcqParams& P, const OutHyp* hyp_h, const ChunkBuffers& cb, int64_t Nvalid, bool first,
+                       uint8_t* flags, cudaStream_t st) {
+  if (Nvalid <= 0) return 0;
+  if (P.m > MAXM) {
+    set_error("prune bound: m exceeds MAXM");
+    return BOCF_ERR_UNSUPPORTED;
+  }
+  const unsigned grid = (unsigned)ceil_div(Nvalid, (int64_t)PB_WARPS * PB_MCB);
+  const int pi = (P.variant == BOCF_ACQ_PI_CF) ? 1 : 0;
+  ProfScope ps("prune_bound_kernel", st);
+#define BOCF_PB(C)                                                                                                     \
+  prune_bound_kernel<C><<<grid, PB_WARPS * 32, 0, st>>>(cb.mean, cb.Nc, Nvalid, P.m, hyp_h, P.Zt, P.S, P.theta, P.L, P.p, \
+                                                       P.fstar, pi, first ? 1 : 0, flags)
+  switch (P.composite) {
+    case BOCF_U_SUMSQ_TARGET: BOCF_PB(BOCF_U_SUMSQ_TARGET); break;
+    case BOCF_U_ROSEN_COMPOSITE: BOCF_PB(BOCF_U_ROSEN_COMPOSITE); break;
+    case BOCF_U_NEG_SUM_EXP: BOCF_PB(BOCF_U_NEG_SUM_EXP); break;
+    case BOCF_U_LINEAR: BOCF_PB(BOCF_U_LINEAR); break;
+    default: set_error("prune bound: no closed-form segment maximum for this composite"); return BOCF_ERR_UNSUPPORTED;
+  }
+#undef BOCF_PB
+  BOCF_LAUNCH_OK("prune_bound_kernel");
+  return 0;
+}
+
+// Survivor list: the indices i < N with flags[i] != 0, ascending, and their number.  Blocks of 256 threads own
+// PL_TILE = 4096 consecutive flags (16 per thread): count -> exclusive scan of the block counts -> write.
+constexpr int PL_THREADS = 256, PL_ITEMS = 16, PL_TILE = PL_THREADS * PL_ITEMS;
+
+// exclusive prefix sum of v over the block (PL_THREADS threads); total into *tot
+__device__ __forceinline__ int pl_block_scan(int v, int* tot) {
+  __shared__ int s_w[PL_THREADS / 32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int incl = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int t = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += t;
+  }
+  if (lane == 31) s_w[warp] = incl;
+  __syncthreads();
+  int before = 0, all = 0;
+#pragma unroll
+  for (int w = 0; w < PL_THREADS / 32; ++w) {
+    const int c = s_w[w];
+    before += (w < warp) ? c : 0;
+    all += c;
+  }
+  *tot = all;
+  return before + incl - v;
+}
+
+__global__ void __launch_bounds__(PL_THREADS) prune_count_kernel(const uint8_t* __restrict__ flags, int64_t N,
+                                                                 int64_t* __restrict__ blk) {
+  const int64_t base = (int64_t)blockIdx.x * PL_TILE + (int64_t)threadIdx.x * PL_ITEMS;
+  int c = 0;
+#pragma unroll
+  for (int k = 0; k < PL_ITEMS; ++k) c += (base + k < N && flags[base + k] != 0) ? 1 : 0;
+  int tot;
+  pl_block_scan(c, &tot);
+  if (threadIdx.x == 0) blk[blockIdx.x] = tot;
+}
+
+// one block: blk[b] <- sum of blk[0 .. b), *count <- sum of all
+__global__ void __launch_bounds__(PL_THREADS) prune_offsets_kernel(int64_t* __restrict__ blk, int nb,
+                                                                   int64_t* __restrict__ count) {
+  __shared__ int64_t s_w[PL_THREADS / 32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int64_t base = 0;
+  for (int b0 = 0; b0 < nb; b0 += PL_THREADS) {
+    const int b = b0 + (int)threadIdx.x;
+    const int64_t v = (b < nb) ? blk[b] : 0;
+    int64_t incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int64_t t = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += t;
+    }
+    if (lane == 31) s_w[warp] = incl;
+    __syncthreads();
+    int64_t before = 0, all = 0;
+#pragma unroll
+    for (int w = 0; w < PL_THREADS / 32; ++w) {
+      before += (w < warp) ? s_w[w] : 0;
+      all += s_w[w];
+    }
+    if (b < nb) blk[b] = base + before + incl - v;
+    base += all;
+    __syncthreads();                                       // s_w is rewritten by the next trip
+  }
+  if (threadIdx.x == 0) *count = base;
+}
+
+__global__ void __launch_bounds__(PL_THREADS) prune_list_kernel(const uint8_t* __restrict__ flags, int64_t N,
+                                                                const int64_t* __restrict__ blk, int64_t* __restrict__ list) {
+  const int64_t base = (int64_t)blockIdx.x * PL_TILE + (int64_t)threadIdx.x * PL_ITEMS;
+  bool f[PL_ITEMS];
+  int c = 0;
+#pragma unroll
+  for (int k = 0; k < PL_ITEMS; ++k) {
+    f[k] = base + k < N && flags[base + k] != 0;
+    c += f[k] ? 1 : 0;
+  }
+  int tot;
+  int64_t pos = blk[blockIdx.x] + pl_block_scan(c, &tot);
+#pragma unroll
+  for (int k = 0; k < PL_ITEMS; ++k)
+    if (f[k]) list[pos++] = base + k;
+}
+
+uint64_t prune_list_work_bytes(int64_t N) { return (uint64_t)ceil_div(N, PL_TILE) * sizeof(int64_t); }
+
+int launch_prune_list(const uint8_t* flags, int64_t N, int64_t* list, int64_t* count, void* work, cudaStream_t st) {
+  const int nb = (int)ceil_div(N, PL_TILE);
+  int64_t* blk = reinterpret_cast<int64_t*>(work);
+  ProfScope ps("prune_list_kernel", st);
+  prune_count_kernel<<<nb, PL_THREADS, 0, st>>>(flags, N, blk);
+  BOCF_LAUNCH_OK("prune_count_kernel");
+  prune_offsets_kernel<<<1, PL_THREADS, 0, st>>>(blk, nb, count);
+  BOCF_LAUNCH_OK("prune_offsets_kernel");
+  if (list) {
+    prune_list_kernel<<<nb, PL_THREADS, 0, st>>>(flags, N, blk, list);
+    BOCF_LAUNCH_OK("prune_list_kernel");
+  }
+  return 0;
+}
+
+// Xg[k] = Xc[list[min(k, last)]] for k < cnt (rows past the last survivor repeat it)
+__global__ void prune_gather_kernel(const double* __restrict__ Xc, int d, const int64_t* __restrict__ list, int64_t last,
+                                    int64_t cnt, double* __restrict__ Xg) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= cnt * d) return;
+  const int64_t k = idx / d;
+  const int q = (int)(idx - k * d);
+  Xg[idx] = Xc[list[min(k, last)] * d + q];
+}
+
+// acq[list[k]] = acq_c[k], dacq[list[k]][.] = dacq_c[k][.] for k < cnt
+__global__ void prune_scatter_kernel(const double* __restrict__ acq_c, const double* __restrict__ dacq_c,
+                                     const int64_t* __restrict__ list, int64_t cnt, int d, double* __restrict__ acq,
+                                     double* __restrict__ dacq) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= cnt * (d + 1)) return;
+  const int64_t k = idx / (d + 1);
+  const int q = (int)(idx - k * (d + 1));
+  const int64_t i = list[k];
+  if (q == d) acq[i] = acq_c[k];
+  else if (dacq) dacq[i * d + q] = dacq_c[k * d + q];
+}
+
+// pruned candidates: acq = 0, dacq = 0
+__global__ void prune_zero_kernel(const uint8_t* __restrict__ flags, int64_t N, int d, double* __restrict__ acq,
+                                  double* __restrict__ dacq) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= N * (d + 1)) return;
+  const int64_t i = idx / (d + 1);
+  const int q = (int)(idx - i * (d + 1));
+  if (flags[i] != 0) return;
+  if (q == d) acq[i] = 0.0;
+  else if (dacq) dacq[i * d + q] = 0.0;
+}
+
+int launch_prune_gather(const double* Xc, int d, const int64_t* list, int64_t last, int64_t cnt, double* Xg,
+                        cudaStream_t st) {
+  ProfScope ps("prune_gather_scatter_kernel", st);
+  prune_gather_kernel<<<(unsigned)ceil_div(cnt * d, 256), 256, 0, st>>>(Xc, d, list, last, cnt, Xg);
+  BOCF_LAUNCH_OK("prune_gather_kernel");
+  return 0;
+}
+
+int launch_prune_scatter(const double* acq_c, const double* dacq_c, const int64_t* list, int64_t cnt, int d, double* acq,
+                         double* dacq, cudaStream_t st) {
+  ProfScope ps("prune_gather_scatter_kernel", st);
+  prune_scatter_kernel<<<(unsigned)ceil_div(cnt * (d + 1), 256), 256, 0, st>>>(acq_c, dacq_c, list, cnt, d, acq, dacq);
+  BOCF_LAUNCH_OK("prune_scatter_kernel");
+  return 0;
+}
+
+int launch_prune_zero(const uint8_t* flags, int64_t N, int d, double* acq, double* dacq, cudaStream_t st) {
+  ProfScope ps("prune_gather_scatter_kernel", st);
+  prune_zero_kernel<<<(unsigned)ceil_div(N * (d + 1), 256), 256, 0, st>>>(flags, N, d, acq, dacq);
+  BOCF_LAUNCH_OK("prune_zero_kernel");
   return 0;
 }
 

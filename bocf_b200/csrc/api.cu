@@ -370,10 +370,21 @@ int bocf_model_destroy(bocf_model* M) {
   if (M->par_host) cudaFreeHost(M->par_host);
   if (M->par_dev) cudaFree(M->par_dev);
   if (M->io_buf) cudaFree(M->io_buf);
+  if (M->prune_count_host) cudaFreeHost(M->prune_count_host);
   if (M->gs.side) cudaStreamDestroy(M->gs.side);
   if (M->gs.fork) cudaEventDestroy(M->gs.fork);
   if (M->gs.join) cudaEventDestroy(M->gs.join);
   delete M;
+  return 0;
+}
+
+int bocf_model_sweep_stats(const bocf_model* M, int64_t* candidates, int64_t* swept) {
+  if (!M || !candidates || !swept) {
+    set_error("bocf_model_sweep_stats: invalid arguments");
+    return BOCF_ERR_INVALID;
+  }
+  *candidates = M->swept_candidates;
+  *swept = M->swept_survivors;
   return 0;
 }
 
@@ -653,8 +664,10 @@ int bocf_posterior(bocf_model* M, int h, const double* Xc, int64_t N, int noisel
   carve_chunk(M, M->scratch, Nc, grad, &cb);
   for (int64_t off = 0; off < N; off += Nc) {
     const int64_t cnt = (N - off < Nc) ? N - off : Nc;
-    if (int rc = launch_posterior_chunk(M, h, Xc + off * M->d, cnt, grad, noiseless, cb, st, var != nullptr,
-                                        dvar != nullptr))
+    // the mean alone: the mean-only K* pass (bitwise the same mean, nothing else written)
+    if (int rc = (var || grad) ? launch_posterior_chunk(M, h, Xc + off * M->d, cnt, grad, noiseless, cb, st, var != nullptr,
+                                                        dvar != nullptr)
+                               : launch_posterior_mean_chunk(M, h, Xc + off * M->d, cnt, cb, st))
       return rc;
     if (int rc = scatter_out(cb.mean, Nc, mean, N, off, cnt, M->m, 1, st)) return rc;
     if (var)
@@ -680,6 +693,24 @@ int bocf_posterior_cov_point(bocf_model* M, int h, const double* Xc, int64_t N, 
   if (int rc = ensure_scratch(M, sizeof(double) * 3 * (size_t)M->m * M->n_pad + 256)) return rc;
   return launch_cov_point(M, h, Xc, N, x2, cov, dcov, reinterpret_cast<double*>(M->scratch), st);
 }
+
+// Pruned sweep.  EI-CF and PI-CF are exactly zero, with a zero gradient, at a candidate none of whose base samples can
+// beat the incumbent, and with uniformly spread candidates that is nearly all of them.  For composites whose maximum over
+// a segment has a closed form, prune_bound_kernel (acq.cu) proves it from the posterior mean alone.  A call of at least
+// PRUNE_MIN_N candidates then runs, chunk by chunk and for every hyper-sample, the mean-only K* pass and the bound over
+// all candidates; lists the survivors on the device and reads their number (one stream synchronisation); and runs the
+// unchanged chunk x hyper-sample sweep over the survivors, gathered into dense chunks of the size the full sweep uses, and
+// scatters the results, zeros elsewhere.  Each survivor's result is bitwise the full sweep's, since no kernel's result for
+// a candidate depends on where in its chunk it sits, with two exceptions that the sweep avoids: the chunk size, which sets
+// the partial-sum split of the contractions, and a chunk of <= 128 candidates, which the MC pass and the gradient sum take
+// through their latency-bound variants (the survivors' last chunk is padded past that; candidates that sit in such a
+// last chunk in the full sweep can differ from it in the last bits).  The first chunk is a probe with a second
+// synchronisation: when it keeps more than PRUNE_KEEP_MAX of its candidates (a pool concentrated near the incumbent) the
+// call runs the full sweep and has lost only the probe.  Smaller calls, such as the acquisition optimiser's L-BFGS rounds
+// of <= 128 candidates, never pay the synchronisations.
+constexpr int64_t PRUNE_MIN_N = 16384;
+constexpr double PRUNE_KEEP_MAX = 0.5;
+static_assert(CAND_TILE > 128, "a survivor chunk padded to 129 candidates must fit the smallest chunk pick_chunk returns");
 
 int bocf_acq_eval(bocf_model* M, int variant, int composite, const double* Xc, int64_t N, const double* Zt, int S,
                   const double* theta, int L, int p, const double* weight, const double* fstar, int H_use,
@@ -726,6 +757,8 @@ int bocf_acq_eval(bocf_model* M, int variant, int composite, const double* Xc, i
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (int rc = resolve_precision(M, st)) return rc;
   const bool grad = (dacq != nullptr);
+  M->swept_candidates = N;
+  M->swept_survivors = N;
 
   // small host-side parameters (theta, weights, f*): staged through a handle-owned ring of PINNED slots and copied
   // to a matching ring of device slots, so the call never synchronises the stream (the L-BFGS rounds of the acquisition
@@ -735,7 +768,16 @@ int bocf_acq_eval(bocf_model* M, int variant, int composite, const double* Xc, i
   const size_t par_doubles = n_theta + (size_t)L + (size_t)H_use * L;
   const int64_t Nc = pick_chunk(M, N, grad, 0);
   const uint64_t chunk_bytes = chunk_bytes_per_candidate(M, grad, Nc) * Nc + kstar_part_bytes(M, Nc) + (1 << 16);
-  if (int rc = ensure_scratch(M, chunk_bytes + 256)) return rc;
+  const int d = M->d;
+  bool prune = N >= PRUNE_MIN_N && prune_supported(variant, composite);
+  for (int l = 0; l < L && prune; ++l) prune = std::isfinite(weight[l]);   // the full sweep's 0 * weight would be a NaN
+  // pruned sweep, on top of the chunk: survivor flags, list-scan blocks, count, survivor list (N of each), gathered
+  // candidates and compacted results (one chunk)
+  const int64_t b_flags = round_up(N, 256), b_work = round_up((int64_t)prune_list_work_bytes(N), 256), b_count = 256;
+  const int64_t b_list = round_up(N * 8, 256), b_x = Nc * d * 8, b_acq = Nc * 8, b_dacq = grad ? Nc * d * 8 : 0;
+  const uint64_t prune_bytes = prune ? (uint64_t)(b_flags + b_work + b_count + b_list + b_x + b_acq + b_dacq) : 0;
+  const uint64_t prune_off = (uint64_t)round_up((int64_t)chunk_bytes, 256);
+  if (int rc = ensure_scratch(M, prune_off + prune_bytes + 256)) return rc;
   ChunkBuffers cb;
   carve_chunk(M, M->scratch, Nc, grad, &cb);
   double* par = nullptr;
@@ -769,20 +811,70 @@ int bocf_acq_eval(bocf_model* M, int variant, int composite, const double* Xc, i
   const bool fused = grad && M->S > 0 &&
                      (variant == BOCF_ACQ_EI_CF || variant == BOCF_ACQ_MEAN_UTILITY ||
                       ((variant == BOCF_ACQ_MA_EI || variant == BOCF_ACQ_MA_PI) && M->m <= 16));
-  for (int64_t off = 0; off < N; off += Nc) {
-    const int64_t cnt = (N - off < Nc) ? N - off : Nc;
+  // cnt candidates X (one chunk) through every hyper-sample into a, g
+  auto sweep = [&](const double* X, int64_t cnt, double* a, double* g) -> int {
     for (int h = 0; h < H_use; ++h) {
       P.fstar = par + n_theta + L + (size_t)h * L;
       P.accumulate = (h > 0) ? 1 : 0;
       if (fused) {
-        if (int rc = launch_fused_grad_chunk(M, h, Xc + off * M->d, cnt, marginal ? 1 : 0, cb, P, acq + off, dacq + off * M->d, st))
-          return rc;
+        if (int rc = launch_fused_grad_chunk(M, h, X, cnt, marginal ? 1 : 0, cb, P, a, g, st)) return rc;
         continue;
       }
-      if (int rc = launch_posterior_chunk(M, h, Xc + off * M->d, cnt, grad, marginal ? 1 : 0, cb, st, !mean_only, !mean_only))
-        return rc;
-      if (int rc = launch_acq_chunk(P, cb, cnt, acq + off, grad ? dacq + off * M->d : nullptr, st)) return rc;
+      if (int rc = launch_posterior_chunk(M, h, X, cnt, grad, marginal ? 1 : 0, cb, st, !mean_only, !mean_only)) return rc;
+      if (int rc = launch_acq_chunk(P, cb, cnt, a, g, st)) return rc;
     }
+    return 0;
+  };
+  if (prune) {
+    char* base = reinterpret_cast<char*>(M->scratch) + prune_off;
+    uint8_t* flags = reinterpret_cast<uint8_t*>(base);
+    void* work = base + b_flags;
+    int64_t* count = reinterpret_cast<int64_t*>(base + b_flags + b_work);
+    int64_t* list = reinterpret_cast<int64_t*>(base + b_flags + b_work + b_count);
+    double* Xg = reinterpret_cast<double*>(base + b_flags + b_work + b_count + b_list);
+    double* acq_c = Xg + Nc * d;
+    double* dacq_c = grad ? acq_c + Nc : nullptr;
+    if (!M->prune_count_host)
+      BOCF_CUDA_OK(cudaHostAlloc(reinterpret_cast<void**>(&M->prune_count_host), sizeof(int64_t), cudaHostAllocDefault));
+    auto bound = [&](int64_t off, int64_t cnt) -> int {
+      for (int h = 0; h < H_use; ++h) {
+        P.fstar = par + n_theta + L + (size_t)h * L;
+        if (int rc = launch_posterior_mean_chunk(M, h, Xc + off * d, cnt, cb, st)) return rc;
+        if (int rc = launch_prune_bound(P, M->hyp + (size_t)h * M->m, cb, cnt, h == 0, flags + off, st)) return rc;
+      }
+      return 0;
+    };
+    auto survivors = [&](int64_t n, int64_t* out_list, int64_t* kept) -> int {
+      if (int rc = launch_prune_list(flags, n, out_list, count, work, st)) return rc;
+      BOCF_CUDA_OK(cudaMemcpyAsync(M->prune_count_host, count, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+      BOCF_CUDA_OK(cudaStreamSynchronize(st));
+      *kept = *M->prune_count_host;
+      return 0;
+    };
+    const int64_t n0 = std::min(N, Nc);
+    int64_t kept = 0;
+    if (int rc = bound(0, n0)) return rc;
+    if (int rc = survivors(n0, nullptr, &kept)) return rc;
+    prune = kept <= PRUNE_KEEP_MAX * (double)n0;
+    if (prune) {
+      for (int64_t off = n0; off < N; off += Nc)
+        if (int rc = bound(off, std::min(Nc, N - off))) return rc;
+      if (int rc = survivors(N, list, &kept)) return rc;
+      M->swept_survivors = kept;
+      if (int rc = launch_prune_zero(flags, N, d, acq, dacq, st)) return rc;
+      for (int64_t off = 0; off < kept; off += Nc) {
+        const int64_t cnt = std::min(Nc, kept - off);
+        const int64_t run = (cnt <= 128) ? 129 : cnt;     // fits: Nc >= CAND_TILE > 128 (pick_chunk, static_assert)
+        if (int rc = launch_prune_gather(Xc, d, list + off, kept - 1 - off, run, Xg, st)) return rc;
+        if (int rc = sweep(Xg, run, acq_c, dacq_c)) return rc;
+        if (int rc = launch_prune_scatter(acq_c, dacq_c, list + off, cnt, d, acq, dacq, st)) return rc;
+      }
+      return 0;
+    }
+  }
+  for (int64_t off = 0; off < N; off += Nc) {
+    const int64_t cnt = (N - off < Nc) ? N - off : Nc;
+    if (int rc = sweep(Xc + off * d, cnt, acq + off, grad ? dacq + off * d : nullptr)) return rc;
   }
   return 0;
 }

@@ -70,6 +70,9 @@ struct bocf_model {
   cudaEvent_t par_event[PAR_SLOTS] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   double* io_buf = nullptr;   // grow-only staging of bocf_acq_eval_host (candidates in, acq / gradient out)
   size_t io_doubles = 0;
+  int64_t* prune_count_host = nullptr;   // pinned: survivor count of the pruned sweep (bocf_acq_eval)
+  int64_t swept_candidates = 0;          // latest bocf_acq_eval: candidates, and those the sweep evaluated (the rest
+  int64_t swept_survivors = 0;           // were proven inactive)
 
   void* scratch = nullptr;
   uint64_t scratch_bytes = 0;
@@ -170,6 +173,10 @@ void carve_chunk(const bocf_model* M, void* base, int64_t Nc, bool grad, ChunkBu
 // noiseless: 0 = likelihood variance added, clipped at 1e-10; 1 = noiseless, clipped; 2 = noiseless, not clipped
 int launch_posterior_chunk(bocf_model* M, int h, const double* Xc, int64_t Nvalid, bool grad, int noiseless,
                            const ChunkBuffers& cb, cudaStream_t st, bool need_var = true, bool need_dvar = true);
+// Posterior mean of hyper-sample h only, into cb.mean: bitwise the mean launch_posterior_chunk / launch_fused_grad_chunk
+// form for the same candidate (no K*, digit planes or G* are written)
+int launch_posterior_mean_chunk(bocf_model* M, int h, const double* Xc, int64_t Nvalid, const ChunkBuffers& cb,
+                                cudaStream_t st);
 
 // ---- split_gemm.cu ------------------------------------------------------------------------------
 int split_scheme_for_slices(int S);                 // 3..6 digit planes -> scheme code (331, 442, 554, 665)
@@ -211,6 +218,21 @@ int launch_fused_grad_chunk(bocf_model* M, int h, const double* Xc, int64_t Nval
                             AcqParams P, double* acq, double* dacq, cudaStream_t st);
 int launch_acq_chunk(const AcqParams& P, const ChunkBuffers& cb, int64_t Nvalid, double* acq, double* dacq,
                      cudaStream_t st);
+// Pruned EI-CF / PI-CF sweep (bocf_acq_eval).  prune_supported: variant and composite have the closed-form bound.
+bool prune_supported(int variant, int composite);
+// flags[i] (first: =, else |=) 1 unless candidate i < Nvalid of the chunk provably has a zero acquisition under the
+// hyper-sample whose mean is in cb.mean, hyp_h = M->hyp + h m and P.fstar
+int launch_prune_bound(const AcqParams& P, const OutHyp* hyp_h, const ChunkBuffers& cb, int64_t Nvalid, bool first,
+                       uint8_t* flags, cudaStream_t st);
+// ascending indices of the non-zero flags[0 .. N) into list (skipped when NULL), their number into *count [dev];
+// work: prune_list_work_bytes(N)
+uint64_t prune_list_work_bytes(int64_t N);
+int launch_prune_list(const uint8_t* flags, int64_t N, int64_t* list, int64_t* count, void* work, cudaStream_t st);
+int launch_prune_gather(const double* Xc, int d, const int64_t* list, int64_t last, int64_t cnt, double* Xg,
+                        cudaStream_t st);
+int launch_prune_scatter(const double* acq_c, const double* dacq_c, const int64_t* list, int64_t cnt, int d, double* acq,
+                         double* dacq, cudaStream_t st);
+int launch_prune_zero(const uint8_t* flags, int64_t N, int d, double* acq, double* dacq, cudaStream_t st);
 // grad: out (L x m x N) = dU/dy_j instead of U
 int launch_utility_eval(int composite, int m, const double* Y, int64_t N, const double* theta, int L, int p,
                         double* out, bool grad, cudaStream_t st);

@@ -48,7 +48,9 @@ struct SplitOut {
   int KCH, S;
 };
 
-// SPL: 0 = fp64 K* output; 5 = exactly five digit planes (the common case, fewer registers); 6 = up to six (so.S)
+// SPL: 0 = fp64 K* output; 5 = exactly five digit planes (the common case, fewer registers); 6 = up to six (so.S);
+//      -1 = no K* output at all: the mean-only pass that decides which candidates the acquisition sweep can skip (api.cu).
+//      Every instantiation forms mu with the same per-pair arithmetic in the same order, so mu is bitwise the same.
 // GRAD: 0 = value quantities only; 1 = also G* and the mean gradient; 2 = G* only -- the fused acquisition-gradient path
 //       (api.cu) folds the mean-gradient contraction into the second contraction's epilogue, which saves the d + 2
 //       fp64 operations per (candidate, training point) the mean gradient costs here.
@@ -102,7 +104,7 @@ __global__ void __launch_bounds__(128, 1) kstar_kernel(const double* __restrict_
   const double* alpha = alphaAll + (int64_t)hj * n_pad;
   constexpr bool SPLIT = SPL > 0;
   constexpr bool GFOLD = SPLIT && GRAD == 2;
-  double* Kout = SPLIT ? nullptr : KsT + (int64_t)j * n16 * Nc;
+  double* Kout = (SPL == 0) ? KsT + (int64_t)j * n16 * Nc : nullptr;
   double* Gout = GRAD ? GsT + (int64_t)j * n16 * Nc : nullptr;
   // split mode: digit planes of this block's 128 candidates (row = tid) for output j
   constexpr int MAXS = SPLIT ? SPL : 1;
@@ -134,7 +136,7 @@ __global__ void __launch_bounds__(128, 1) kstar_kernel(const double* __restrict_
     const int bmax = min(128, n16 - b0);
     // 16 (split: one 16-byte piece of a digit-plane row) or 4 training points per trip, evaluated branch-free so the
     // independent chains interleave; padded points b >= n are evaluated like the others and masked at the end
-    constexpr int UNR = SPLIT ? 16 : 4;
+    constexpr int UNR = (SPL != 0) ? 16 : 4;
     for (int bb0 = 0; bb0 < bmax; bb0 += UNR) {
       unsigned long long dg4[4];
 #pragma unroll
@@ -183,9 +185,9 @@ __global__ void __launch_bounds__(128, 1) kstar_kernel(const double* __restrict_
           }
         }
         if (GRAD) Gout[(int64_t)b * Nc + i] = SPLIT ? gv * sgcs[bb] : gv;
-        if (!SPLIT) {
+        if (SPL == 0) {
           Kout[(int64_t)b * Nc + i] = kv;
-        } else {
+        } else if (SPLIT) {
           dg4[e & 3] = (unsigned long long)__double_as_longlong(fma(kv, aq, magicb));
           if ((e & 3) == 3) {                                     // byte transpose of four points' digits
             uint32_t o[MAXS];
@@ -509,7 +511,8 @@ static int launch_kstar_t(bocf_model* M, int h, const double* Xc, int64_t Nvalid
   kstar_kernel<KIND, DP, G, SP><<<kgrid, 128, 0, st>>>(Xc, Nvalid, cb.Nc, M->d, M->n, M->n16, M->n_pad, M->m, h, M->hyp, \
                                                        M->Xs, M->xsq, M->alpha, cb.KsT, cb.GsT, mean_out, dmean_out, so,     \
                                                        run.j0)
-  if (grad == 2 && spl == 5) BOCF_KSTAR(2, 5);
+  if (grad < 0) BOCF_KSTAR(0, -1);
+  else if (grad == 2 && spl == 5) BOCF_KSTAR(2, 5);
   else if (grad == 2 && spl == 6) BOCF_KSTAR(2, 6);
   else if (grad && spl == 5) BOCF_KSTAR(1, 5);
   else if (grad && spl == 6) BOCF_KSTAR(1, 6);
@@ -534,9 +537,10 @@ static int launch_kstar_k(bocf_model* M, int h, const double* Xc, int64_t Nvalid
   return launch_kstar_t<KIND, MAXD>(M, h, Xc, Nvalid, grad, cb, run, st);
 }
 
+// grad: -1 = mean only (launch_posterior_mean_chunk); 0 / 1 / 2 = kstar_kernel's GRAD
 static int launch_kstar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, int grad, const ChunkBuffers& cb,
                         cudaStream_t st) {
-  ProfScope ps("kstar_kernel", st);
+  ProfScope ps(grad < 0 ? "kstar_mean_kernel" : "kstar_kernel", st);
   // one launch per run of outputs that share a kernel family (one launch when they all do)
   const int rc = for_each_kind_run(M, [&](int kind, OutRun run) -> int {
     switch (kind) {
@@ -559,6 +563,11 @@ static int launch_kstar(bocf_model* M, int h, const double* Xc, int64_t Nvalid, 
     BOCF_LAUNCH_OK("kstar_reduce_kernel");
   }
   return 0;
+}
+
+int launch_posterior_mean_chunk(bocf_model* M, int h, const double* Xc, int64_t Nvalid, const ChunkBuffers& cb,
+                                cudaStream_t st) {
+  return launch_kstar(M, h, Xc, Nvalid, -1, cb, st);
 }
 
 // ===================================================================================================

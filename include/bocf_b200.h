@@ -159,6 +159,10 @@ int bocf_model_get_factor(bocf_model* mdl, int h, int j, double* L, double* Linv
 /* Candidates the library evaluates per internal chunk for a call with N candidates (the K* / V scratch of one chunk
  * must fit the scratch limit); results never depend on it -- exposed so tests can place spot checks on chunk borders. */
 int64_t bocf_model_chunk_candidates(bocf_model* mdl, int64_t N, int with_grad);
+
+/* Of the latest bocf_acq_eval on the handle: the candidates, and how many of them the sweep evaluated.  Fewer when the
+ * posterior mean proved the others' EI-CF / PI-CF exactly zero (pruned sweep); equal when the full sweep ran. */
+int bocf_model_sweep_stats(const bocf_model* mdl, int64_t* candidates, int64_t* swept);
 int bocf_model_n(const bocf_model* mdl);
 int bocf_model_H(const bocf_model* mdl);
 
@@ -179,7 +183,10 @@ int bocf_model_active_scheme(bocf_model* mdl);
 int bocf_debug_split_gemm(const double* A, const double* B, int R, int N, int K, int slices, int tri, double* out,
                           void* stream);
 
-/* Upper bound, in bytes, of the handle's internal scratch (default 4 GiB). */
+/* Upper bound, in bytes, of the handle's per-chunk candidate scratch (default 4 GiB): it sets the chunk size of the
+ * sweeps.  A pruned EI-CF / PI-CF sweep (bocf_acq_eval) adds, on top of it, 9 bytes per candidate of the call (survivor
+ * flags and list) and one chunk of gathered candidates and results; it never changes the chunk size, so that a
+ * candidate's result is the same whether the call was pruned or not. */
 int bocf_model_set_scratch_limit(bocf_model* mdl, uint64_t bytes);
 
 /* Posterior of hyper-sample h at N candidates Xc [dev] N x d.  Outputs [dev], any may be NULL:

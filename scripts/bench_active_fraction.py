@@ -9,11 +9,15 @@ The fused gradient walks only the units (output, 128-candidate tile) with a non-
 Each build runs in its own process (BOCF_LIB_PATH); builds alternate for --rounds rounds.  Steps are timed with CUDA
 events and a 256 MiB L2 flush between steps.  `active_tiles` is the share of 128-candidate tiles with a non-zero EI,
 read from the outputs after the timed steps: for sumsq_target every output of an improving candidate has a non-zero
-weight, so it is the share of units the second contraction walks.
+weight, so it is the share of units the second contraction walks.  `kernel_ms` are the library's per-kernel CUDA-event
+times per step, from a separate profiled pass.  `pruned` is the share of the candidates the library proved inactive
+from the posterior mean and left out of the sweep (bocf_model_sweep_stats; null for a build without it).  A library at
+<tree>/bocf_b200/csrc/ runs with the Python package of <tree>, so builds with different bindings can be compared.
 
     python scripts/bench_active_fraction.py --libs parent.so branch.so [--rounds 2] [--steps 3] [--warmup 2]
 """
 import argparse
+import ctypes
 import json
 import os
 import subprocess
@@ -36,7 +40,20 @@ def candidate_sets():
     return {"uniform": uniform, "focused": focused, "mix": mix}
 
 
+def pruned_share(model):
+    """1 - swept / candidates of the model's latest acquisition call, as the library counted them."""
+    fn = getattr(model._lib, "bocf_model_sweep_stats", None)
+    if fn is None:
+        return None
+    n, kept = ctypes.c_int64(0), ctypes.c_int64(0)
+    fn(model._handle, ctypes.byref(n), ctypes.byref(kept))
+    return 1.0 - kept.value / n.value
+
+
 def child(args):
+    tree = os.path.dirname(os.path.dirname(os.path.dirname(os.environ.get("BOCF_LIB_PATH", ""))))
+    if os.path.exists(os.path.join(tree, "bocf_b200", "__init__.py")):
+        sys.path.insert(0, tree)
     import torch
     import bocf_b200
     from bocf_b200 import _lib
@@ -65,11 +82,19 @@ def child(args):
             flush.zero_()
             torch.cuda.synchronize()
             ms.append(e0.elapsed_time(e1))
+        pruned = pruned_share(model)
+        _lib.profile_enable(True)
+        for _ in range(args.steps):
+            acq._compute_acq_withGradients(Xd)
+            flush.zero_()
+        prof = _lib.profile_report()
+        _lib.profile_enable(False)
         act = (a.reshape(-1) > 0).cpu().numpy()
         tiles = np.zeros(-(-N // 128), dtype=bool)
         np.logical_or.at(tiles, np.arange(N) // 128, act)
         out[name] = {"ms_per_step": float(np.median(ms)), "ms": ms, "active_candidates": float(act.mean()),
-                     "active_tiles": float(tiles.mean())}
+                     "active_tiles": float(tiles.mean()), "pruned": pruned,
+                     "kernel_ms": {k: v[1] / args.steps for k, v in sorted(prof.items())}}
         del Xd, a, g
     print(json.dumps(out))
 
