@@ -25,11 +25,11 @@ EXPORTS = [
     "bocf_model_set_precision", "bocf_model_active_slices", "bocf_model_active_scheme", "bocf_model_chunk_candidates", "bocf_model_sweep_stats", "bocf_debug_split_gemm", "bocf_model_log_likelihood", "bocf_model_append_point",
 ]
 # name -> (enum bocf_precision, slices).  "splitN": both contractions on the N-plane scheme; "splitNM": variance on N,
-# variance gradient on M <= N planes (include/bocf_b200.h).
+# variance gradient on M = N or N - 1 >= 3 planes, the pairs the library accepts (include/bocf_b200.h).
 PRECISIONS = {"fp64": (0, 0), "auto": (2, 0), "mixed": (3, 0)}
 for _s1 in range(3, 7):
     PRECISIONS["split%d" % _s1] = (1, _s1)
-    for _s2 in range(3, _s1 + 1):
+    for _s2 in range(max(3, _s1 - 1), _s1 + 1):
         PRECISIONS["split%d%d" % (_s1, _s2)] = (1, 10 * _s1 + _s2)
 
 

@@ -155,6 +155,12 @@ static int apply_precision(bocf_model* M, cudaStream_t st) {
   return split_prepare(M, sch1, sch2, st);
 }
 
+// The split-integer plane pairs the first contraction is instantiated for (split_gemm.cu launch_var): the variance on
+// s1 = 3..6 digit planes, its gradient on s2 = s1 or s1 - 1 >= 3 planes (s2 = 0: s1).
+static bool split_pair_supported(int s1, int s2) {
+  return s1 >= 3 && s1 <= 6 && (s2 == 0 || s2 == s1 || (s2 == s1 - 1 && s2 >= 3));
+}
+
 static int resolve_precision(bocf_model* M, cudaStream_t st) {
   if (M->precision_resolved) return 0;
   if (int rc = apply_precision(M, st)) return rc;
@@ -266,6 +272,24 @@ int bocf_model_create(bocf_model** out, int m, int d, int kernel, int device) {
     set_error("bocf_model_create: invalid arguments (need m >= 1, 1 <= d <= 16, known kernel)");
     return BOCF_ERR_INVALID;
   }
+  int precision = BOCF_PREC_AUTO, s1 = 0, s2 = 0;               // library default
+  if (const char* env = std::getenv("BOCF_PRECISION")) {      // fp64 | auto | mixed | split3 .. split6 | split<s1><s2>
+    const std::string v(env);
+    const auto digit = [&](size_t k) { return (v.size() > k && v[k] >= '0' && v[k] <= '9') ? v[k] - '0' : -1; };
+    if (v == "auto" || v.empty()) precision = BOCF_PREC_AUTO;
+    else if (v == "mixed") precision = BOCF_PREC_MIXED;
+    else if (v == "fp64") precision = BOCF_PREC_FP64_DMMA;
+    else if (v.rfind("split", 0) == 0 && (v.size() == 6 || (v.size() == 7 && digit(6) > 0)) &&
+             split_pair_supported(digit(5), v.size() == 7 ? digit(6) : 0)) {
+      precision = BOCF_PREC_SPLIT_I8;
+      s1 = digit(5);
+      s2 = v.size() == 7 ? digit(6) : 0;
+    } else {
+      set_error("bocf_model_create: BOCF_PRECISION=" + v + " is not one of fp64, auto, mixed, split3 .. split6 or "
+                "split<s1><s2> with 3 <= s1 <= 6 and s2 = s1 or s1 - 1 >= 3");
+      return BOCF_ERR_INVALID;
+    }
+  }
   int ndev = 0;
   BOCF_CUDA_OK(cudaGetDeviceCount(&ndev));
   if (device < 0 || device >= ndev) {
@@ -282,17 +306,10 @@ int bocf_model_create(bocf_model** out, int m, int d, int kernel, int device) {
   M->kernel = kernel;
   M->kinds.assign((size_t)m, kernel);
   M->device = device;
-  M->precision = BOCF_PREC_AUTO;                                // library default
-  if (const char* env = std::getenv("BOCF_PRECISION")) {      // fp64 | auto | mixed | split3 .. split6 | split<s1><s2>
-    const std::string v(env);
-    if (v == "auto") M->precision = BOCF_PREC_AUTO;
-    else if (v == "mixed") M->precision = BOCF_PREC_MIXED;
-    else if (v == "fp64") M->precision = BOCF_PREC_FP64_DMMA;
-    else if (v.rfind("split", 0) == 0 && (v.size() == 6 || v.size() == 7) && v[5] >= '3' && v[5] <= '6') {
-      M->precision = BOCF_PREC_SPLIT_I8;
-      M->slices_req = v[5] - '0';
-      M->slices2_req = (v.size() == 7 && v[6] >= '3' && v[6] <= v[5]) ? v[6] - '0' : 0;
-    }
+  M->precision = precision;
+  if (precision == BOCF_PREC_SPLIT_I8) {
+    M->slices_req = s1;
+    M->slices2_req = s2;
   }
   *out = M;
   return 0;
@@ -323,9 +340,9 @@ int bocf_model_set_precision(bocf_model* M, int mode, int slices, void* stream) 
     s2 = slices % 10;
   }
   if (!M || mode < BOCF_PREC_FP64_DMMA || mode > BOCF_PREC_MIXED ||
-      (mode == BOCF_PREC_SPLIT_I8 && (s1 < 3 || s1 > 6 || (s2 != 0 && (s2 < 3 || s2 > s1))))) {
+      (mode == BOCF_PREC_SPLIT_I8 && !split_pair_supported(s1, s2))) {
     set_error("bocf_model_set_precision: mode must be 0 (fp64), 1 (split int8: slices = 3..6, or 10 s1 + s2 with "
-              "3 <= s2 <= s1 <= 6), 2 (auto) or 3 (mixed)");
+              "3 <= s1 <= 6 and s2 = s1 or s1 - 1 >= 3), 2 (auto) or 3 (mixed)");
     return BOCF_ERR_INVALID;
   }
   M->precision = mode;

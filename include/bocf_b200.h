@@ -93,7 +93,8 @@ enum bocf_precision {
   BOCF_PREC_SPLIT_I8 = 1,   /* tcgen05.mma kind::i8: operands split into signed 8-bit digit planes, exact int32
                                accumulation in tensor memory.  `slices` = s (3..6): both contractions use the scheme of
                                s planes (3: 8 digit pairs, 4: 13, 5: 15, 6: 21);  `slices` = 10 s1 + s2: the first
-                               contraction (variance) uses s1, the second (variance gradient) s2 <= s1               */
+                               contraction (variance) uses s1, the second (variance gradient) s2 = s1 or s1 - 1 >= 3
+                               (33, 43, 44, 54, 55, 65, 66); other pairs return BOCF_ERR_INVALID                     */
   BOCF_PREC_AUTO = 2,       /* default: smallest variance scheme whose predicted relative error stays inside the fp64
                                bar (1e-6, element-wise) both away from the data (bound from max|L^-1|) and next to a
                                training input, where the variance drops to the noise level (bound from the smallest
@@ -167,8 +168,9 @@ int bocf_model_n(const bocf_model* mdl);
 int bocf_model_H(const bocf_model* mdl);
 
 /* Select the contraction arithmetic (enum bocf_precision).  May be called before or after bocf_model_factorize; the
- * digit planes of L^-1 are (re)built when needed.  The environment variable BOCF_PRECISION (fp64 | auto | mixed | split3..6 | split<s1><s2>)
- * sets the initial mode of new handles.  The planes are built lazily by the first posterior / acquisition call after a
+ * digit planes of L^-1 are (re)built when needed.  The environment variable BOCF_PRECISION (fp64 | auto | mixed | split3..6 | split<s1><s2>
+ * with a pair set_precision accepts) sets the initial mode of new handles; bocf_model_create returns BOCF_ERR_INVALID
+ * for any other non-empty value.  The planes are built lazily by the first posterior / acquisition call after a
  * factorisation (likelihood-only callers never pay for them).  bocf_model_active_slices: digit planes of the first contraction in use (0 = fp64);
  * bocf_model_active_scheme: 1000 * scheme of the first contraction + scheme of the second, a scheme being
  * 100 SA + 10 SB + LMIN (digit planes of the candidate side, of the factor side, lowest digit-pair weight kept);
